@@ -2,7 +2,7 @@
 """Benchmark of the UCD distillation-loss hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--workload voc|ade|city|sweep:<pixels>] [--batch B]
+                    [--workload voc|ade|city|sweep:<pixels>] [--batch B] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic batch, forward + backward:
   bilinear logit upsample (old model under no_grad first, then the new one: train.py:100-108) -> pre_contrastive_pixel -> PixelConLossV2
@@ -19,6 +19,10 @@ Workloads (BASELINE.json configs; default = configs[1] held on one GPU, which is
 Weak scaling: each rank holds its own images; with N>1 the contrast columns of all ranks are exchanged (one
 all-gather over NCCL, overlapped with the sweep over the local columns) so negatives span the global batch.
 metric = pixel pairs (N_a local x N_c global, summed over ranks) per second, in Mpairs/s.
+
+--dump-outputs DIR writes what the last timed step handed back to its caller (rank 0): the losses and the gradients
+with respect to f_n and the low-res logits, one float32 DIR/<name>.npy each.  Inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import gc
@@ -29,6 +33,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -76,6 +81,24 @@ KERNELS_PER_CALL = {"ucd_upsample_bilinear_fwd": 1, "ucd_upsample_bilinear_bwd":
 HOST_ONLY_CALLS = ("ucd_last_error", "ucd_version", "ucd_device_ok", "ucd_con_max_tiles", "ucd_con_prob_kpad",
                    "ucd_con_num_bins", "ucd_con_px_meta_ints", "ucd_con_blk_meta_ints", "ucd_con_workspace_bytes",
                    "ucd_reduce_scratch_floats", "ucd_seg_fused_workspace_floats")
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, outputs):
+    """One float32 <name>.npy per output.  When the outputs exceed DUMP_BYTES together, every non-scalar one is cut to
+    the same fraction of its elements: a seeded (seed 0), sorted sample of its flattened indices, so that the sample is
+    the same from run to run and from build to build."""
+    os.makedirs(out_dir, exist_ok=True)
+    limit = (DUMP_BYTES - 4096) // 4            # elements; 4 KB left for the .npy headers
+    total = sum(t.numel() for t in outputs.values())
+    for name, t in outputs.items():
+        a = t.detach().float().cpu()
+        if total > limit and a.numel() > 1:
+            keep = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:a.numel() * limit // total]
+            a = a.reshape(-1)[keep.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def gen(seed, *shape, scale=1.0):
@@ -259,7 +282,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the informational legs (N1 / N4 variants, GPU arm at the CPU sample size)")
     ap.add_argument("--no-parity", action="store_true", help="N>1: skip the concatenated-batch parity check on rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the losses and gradients of the last timed step as DIR/<name>.npy (float32, at most "
+                         "64 MB in all: larger outputs are cut to a seeded sample of their elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the ucd_b200 arm; the reference arm runs a smaller sample")
     wl = get_workload(args.workload, args.batch)
     if args.impl == "reference":
         return run_reference(args, wl)
@@ -313,7 +343,7 @@ def main():
         loss = ce + con / 100 + 10 * kd
         loss.backward()
         state.update(n_a=tup[0].shape[0], n_c=tup[1].shape[0], con=con.detach(), ce=ce.detach(), kd=kd.detach(),
-                     g_fn=f_n.grad, g_lr=lr.grad)
+                     loss=loss.detach(), g_fn=f_n.grad, g_lr=lr.grad)
         return loss
 
     def barrier():
@@ -347,6 +377,10 @@ def main():
     ms_dev = timed(lambda: step(devin), args.steps)
     timed_region_s = time.perf_counter() - t_wall0
     clocks = sampler.stop() if (rank == 0 and sampler.thr is not None) else None
+    if args.dump_outputs and rank == 0:
+        names = (("loss", "loss"), ("con", "con"), ("ce", "ce"), ("kd", "kd"), ("grad_f_n", "g_fn"),
+                 ("grad_logits_lr", "g_lr"))
+        dump_outputs(args.dump_outputs, {name: state[key] for name, key in names if key in state})
     # ---- the same loop once more with a CUDA-event pair around every C-ABI call: per-kernel-group device times for
     #      the rooflines and the launch count.  (The ~35 extra event records per step cost host time and stream slots:
     #      this pass runs up to 15 % slower than the plain loop, which is why it is not the headline.) ----

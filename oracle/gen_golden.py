@@ -24,7 +24,8 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, REF)
 warnings.filterwarnings("ignore")
 
-from oracle.ucd_oracle import synthetic_case  # noqa: E402
+from oracle.ucd_oracle import (LABEL_DOWNSAMPLE_SIZES, label_downsample_maps, label_map_digest,  # noqa: E402
+                               synthetic_case)
 from utils.loss import (PixelConLossV2, UnbiasedCrossEntropy,  # noqa: E402  (the reference)
                         UnbiasedKnowledgeDistillationLoss, pre_contrastive_pixel)
 
@@ -199,28 +200,20 @@ def main():
         )
         if name.startswith("tiny"):
             fx.update(full_A=r64["A"].numpy(), full_Cst=r64["Cst"].numpy(), full_P=r64["P"].numpy(),
-                      full_g_fn=r64["g_fn"].numpy(), full_g_lr=r64["g_lr"].numpy(),
-                      full_ce_px=r64["ce_px"].numpy())
+                      full_g_fn=r64["g_fn"].numpy(), full_g_lr=r64["g_lr"].numpy())
         np.savez_compressed(os.path.join(OUT, name + ".npz"), **fx)
         print(f"{name}: N_a={len(fx['la'])} N_c={len(fx['lc'])} sum_la={fx['la'].astype(int).sum()} "
               f"sum_lc={fx['lc'].astype(int).sum()} P1={fx['p_ones'][0]} con={fx['con']} ce={fx['ce']} kd={fx['kd']} "
               f"|g_fn|={fx['g_fn_norm'][0]:.6g} |g_lr|={fx['g_lr_norm'][0]:.6g}")
 
-    # label-downsample vectors: the reference's own resize+cast+clamp on assorted label maps
-    rng = torch.Generator().manual_seed(77)
-    lab_fx = {}
-    for i, (H, W, h, w) in enumerate([(513, 513, 33, 33), (512, 512, 32, 32), (321, 321, 21, 21),
-                                      (500, 375, 32, 24), (512, 1024, 32, 64), (129, 257, 9, 17)]):
-        lab = torch.randint(0, 21, (2, H, W), generator=rng)
-        # coarse blocks so that constant regions (the rounding hazard) exist, plus an ignore band
-        blk = torch.randint(0, 21, (2, H // 37 + 1, W // 29 + 1), generator=rng)
-        lab_b = blk.repeat_interleave(37, 1).repeat_interleave(29, 2)[:, :H, :W].clone()
-        lab_b[:, : H // 20] = 255
-        for tag, L in (("rand", lab), ("block", lab_b)):
-            f_dummy = torch.zeros(2, 4, h, w)
-            _, flat = pre_contrastive_pixel(f_dummy, L)
-            lab_fx[f"{tag}{i}_in"] = L.numpy().astype(np.uint8)
-            lab_fx[f"{tag}{i}_out"] = flat.numpy().astype(np.int8).reshape(2, h, w)
+    # label-downsample vectors: the reference's own resize+cast+clamp on assorted label maps.  The maps themselves are
+    # regenerated from their seed by the tests (stored, they would take 1.7 MB); the fixture keeps their digests.
+    maps, lab_fx = label_downsample_maps(), {}
+    for i, (H, W, h, w) in enumerate(LABEL_DOWNSAMPLE_SIZES):
+        for n in ("rand%d" % i, "block%d" % i):
+            _, flat = pre_contrastive_pixel(torch.zeros(2, 4, h, w), torch.from_numpy(maps[n].astype(np.int64)))
+            lab_fx[n + "_in_sha256"] = np.array(label_map_digest(maps[n]))
+            lab_fx[n + "_out"] = flat.numpy().astype(np.int8).reshape(2, h, w)
     np.savez_compressed(os.path.join(OUT, "label_downsample.npz"), **lab_fx)
     print("label_downsample: ", len(lab_fx) // 2, "maps")
 

@@ -652,3 +652,29 @@ def synthetic_case(B: int, h: int, w: int, H: int, W: int, c_tot: int, c_old: in
         add = proto[cls].permute(0, 3, 1, 2)
         f_n, f_o = 0.3 * f_n + 0.7 * add, 0.3 * f_o + 0.7 * add
     return dict(f_n=f_n, f_o=f_o, l_po=l_po, logits_lr=lr, labels=blob_labels(B, H, W, c_old, c_tot))
+
+
+LABEL_DOWNSAMPLE_SIZES = [(513, 513, 33, 33), (512, 512, 32, 32), (321, 321, 21, 21), (500, 375, 32, 24),
+                          (512, 1024, 32, 64), (129, 257, 9, 17)]   # (H, W, h, w)
+
+
+def label_downsample_maps():
+    """Seeded label maps of the label-downsample fixture (tests/golden/label_downsample.npz), in generation order:
+    {"rand<i>" / "block<i>": uint8 [2, H, W]} for the i-th entry of LABEL_DOWNSAMPLE_SIZES.  "rand" draws every pixel
+    from 0..20; "block" holds constant 37 x 29 blocks (the rounding hazard of the resize) under an ignore band."""
+    rng = torch.Generator().manual_seed(77)
+    maps = {}
+    for i, (H, W, _, _) in enumerate(LABEL_DOWNSAMPLE_SIZES):
+        lab = torch.randint(0, 21, (2, H, W), generator=rng)
+        blk = torch.randint(0, 21, (2, H // 37 + 1, W // 29 + 1), generator=rng)
+        lab_b = blk.repeat_interleave(37, 1).repeat_interleave(29, 2)[:, :H, :W].clone()
+        lab_b[:, : H // 20] = 255
+        maps["rand%d" % i] = lab.numpy().astype(np.uint8)
+        maps["block%d" % i] = lab_b.numpy().astype(np.uint8)
+    return maps
+
+
+def label_map_digest(lab: np.ndarray) -> str:
+    """sha256 of a uint8 label map's bytes (C order): the fixture stores it so that generator drift is caught."""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(lab, dtype=np.uint8).tobytes()).hexdigest()

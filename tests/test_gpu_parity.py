@@ -157,8 +157,12 @@ def test_label_downsample_bit_exact(U, golden_dir):
     """label_n of the prep kernel == the reference's resize+int8+clamp on every golden label map."""
     from ucd_b200.losses import _build_pack
     fx = np.load(os.path.join(golden_dir, "label_downsample.npz"))
-    for n in sorted(k[:-3] for k in fx.files if k.endswith("_in")):
-        lab = torch.from_numpy(fx[n + "_in"].astype(np.int64)).cuda()
+    maps = O.label_downsample_maps()
+    names = sorted(k[:-len("_in_sha256")] for k in fx.files if k.endswith("_in_sha256"))
+    assert len(names) == 12 and sorted(maps) == names
+    for n in names:
+        assert O.label_map_digest(maps[n]) == str(fx[n + "_in_sha256"]), "label map generator drifted: " + n
+        lab = torch.from_numpy(maps[n].astype(np.int64)).cuda()
         want = fx[n + "_out"].astype(np.int64)
         B, h, w = want.shape
         l_po = torch.zeros(B, 2, h, w, device="cuda")
@@ -166,7 +170,7 @@ def test_label_downsample_bit_exact(U, golden_dir):
         f = torch.randn(B, 256, h, w, device="cuda")
         pk = _build_pack(f, f, l_po, lab, 20)
         assert np.array_equal(pk.label_n.view(B, h, w).cpu().numpy().astype(np.int64), want), n
-        assert np.array_equal(pk.label_n.cpu().numpy(), O.downsample_labels(fx[n + "_in"].astype(np.int64), h, w).reshape(-1)), n
+        assert np.array_equal(pk.label_n.cpu().numpy(), O.downsample_labels(maps[n].astype(np.int64), h, w).reshape(-1)), n
 
 
 @pytest.mark.parametrize("name", ["tiny_b2", "voc15-5_b2_513", "voc15-5s_b3_512", "city13-6_b3", "voc15-5s_b2_corr"])
