@@ -113,6 +113,18 @@ int ucd_upsample_bilinear_fwd(const float* in, float* out, int64_t planes, int h
                               void* stream);
 int ucd_upsample_bilinear_bwd(const float* gout, float* gin, int64_t planes, int h, int w, int H, int W,
                               void* stream);
+/* ucd_unce_unkd_bwd contracted with the adjoint of ucd_upsample_bilinear_fwd: when the logits x [B,C,H,W] are the
+ * upsample of lr [B,C,h,w], d_lr [B,C,h,w] = upsample_adjoint(dx) of the dx ucd_unce_unkd_bwd would write (same
+ * per-element values; the adjoint's summation order is its own).  dx is never written: one read-only pass over x, t,
+ * the labels and the saved planes.  d_lr is overwritten.  Deterministic.  UCD_ENOSUP (nothing launched) unless the
+ * shape is one the sweep-form adjoint takes: H % h == 0, W % w == 0, (W / w) % 8 == 0, W / 4 a multiple of 32 and
+ * <= 256, all planes 16-byte aligned; the caller then takes ucd_unce_unkd_bwd + ucd_upsample_bilinear_bwd. */
+int ucd_unce_unkd_bwd_lowres(const float* x, const int64_t* y, const float* lse_all, const float* bkg_gap,
+                             const float* ce_g_px, const float* ce_g_scalar, float ce_g_mul, const float* ce_stats,
+                             int mean_over_valid, int old_cl, int ignore_index, const float* t, const float* mask,
+                             float alpha, const float* lse3, const float* kd_g_px, const float* kd_g_scalar,
+                             float kd_g_mul, int kd_variant, float* d_lr, int B, int C, int C_old, int h, int w, int H,
+                             int W, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * N1 (SURVEY.md 8f), opt-in: upsample + unbiased CE + unbiased KD fused, from the LOW-RES logits

@@ -13,6 +13,8 @@ LIB_PATH = os.path.join(_HERE, "libucd_b200.so")
 
 _lib = None
 
+UCD_ENOSUP = -3   # include/ucd_b200.h: a valid request this entry point does not take (the caller has another path)
+
 P = c_void_p
 _PROTOS = {
     "ucd_version": (c_int, []),
@@ -27,6 +29,8 @@ _PROTOS = {
     "ucd_kd_bwd": (c_int, [P, P, P, c_float, P, P, P, c_float, P, c_int, c_int, c_int, c_int, c_int64, c_int, P]),
     "ucd_unce_unkd_bwd": (c_int, [P, P, P, P, P, P, c_float, P, c_int, c_int, c_int, P, P, c_float, P, P, P, c_float, c_int,
                                   P, c_int, c_int, c_int, c_int, c_int64, P]),
+    "ucd_unce_unkd_bwd_lowres": (c_int, [P, P, P, P, P, P, c_float, P, c_int, c_int, c_int, P, P, c_float, P, P, P,
+                                         c_float, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ucd_bkg_mask": (c_int, [P, P, P, c_int, c_int, c_int64, c_int, P]),
     "ucd_upsample_bilinear_fwd": (c_int, [P, P, c_int64, c_int, c_int, c_int, c_int, P]),
     "ucd_upsample_bilinear_bwd": (c_int, [P, P, c_int64, c_int, c_int, c_int, c_int, P]),

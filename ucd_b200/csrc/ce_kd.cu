@@ -10,6 +10,9 @@
 // element (see lse_push).  Partial sums go to a per-block slot and are reduced by a second
 // fixed-order kernel, so results are run-to-run deterministic.
 #include "common.cuh"
+#include "sweep_adjoint.cuh"
+
+#include <stdlib.h>
 
 namespace ucd {
 
@@ -534,7 +537,90 @@ unkd_bwd_kernel(const float* __restrict__ x, const float* __restrict__ t, const 
 // kernels (the second accumulating) move 2 x + t + 3 dx = 2.5 GB at the BASELINE workload, this one x + t + dx = 1.26 GB.
 //   dx_c = u_ce ( p_c - [y'==0 ? [c<old_cl] p_c e^{lse - lse_old} : [c==y'] ] )           (SURVEY A.3, UNCE)
 //        + u_kd ( p_c - [c in S_b] p_c q_0 e^{lse - lse_b} - [1<=c<C_old] q_c )           (UNKD; S_b = {0} U new)
+// The per-pixel coefficients (pair_coef) and the per-element expression (pair_dx) are shared with the kernel that
+// folds the bilinear adjoint in (unce_unkd_bwd_lowres_kernel): both form bit-identical dx.
 // ------------------------------------------------------------------------------------------
+struct PairArgs {
+  const long long* y;
+  const float *lse_all, *bkg_gap, *ce_g_px, *t, *mask, *lse3, *kd_g_px;
+  long long plane;  // B * HW: stride of the lse3 planes
+  float gs_ce, gs_kd, a2, inv_cold;
+  int old_cl, ignore_index, C, C_old, mask_zero;
+};
+
+__device__ __forceinline__ PairArgs pair_args(const long long* y, const float* lse_all, const float* bkg_gap,
+                                              const float* ce_g_px, const float* ce_g_scalar, float ce_g_mul,
+                                              const float* ce_stats, int mean_over_valid, int old_cl, int ignore_index,
+                                              const float* t, const float* mask, float alpha, const float* lse3,
+                                              const float* kd_g_px, const float* kd_g_scalar, float kd_g_mul,
+                                              int mask_zero, int B, int C, int C_old, long long HW) {
+  PairArgs a;
+  a.y = y, a.lse_all = lse_all, a.bkg_gap = bkg_gap, a.ce_g_px = ce_g_px, a.t = t, a.mask = mask, a.lse3 = lse3;
+  a.kd_g_px = kd_g_px;
+  a.plane = (long long)B * HW;
+  a.a2 = alpha * kLog2e;
+  a.inv_cold = 1.f / (float)C_old;
+  a.gs_ce = 0.f;
+  if (ce_g_px == nullptr) {
+    a.gs_ce = ce_g_scalar[0] * ce_g_mul;
+    if (mean_over_valid) a.gs_ce = a.gs_ce / ce_stats[1];
+  }
+  a.gs_kd = (kd_g_px == nullptr) ? kd_g_scalar[0] * kd_g_mul : 0.f;
+  a.old_cl = old_cl, a.ignore_index = ignore_index, a.C = C, a.C_old = C_old, a.mask_zero = mask_zero;
+  return a;
+}
+
+// per-pixel coefficients of VEC adjacent pixels; px = b * HW + p, tp = t + b * C_old * HW + p (its plane 0: q_0)
+template <int VEC>
+struct PairCoef {
+  float la2[VEC], lt2[VEC], uce[VEC], ukd[VEC], fold[VEC], fb[VEC];
+  int lab[VEC];
+};
+
+template <int VEC>
+__device__ __forceinline__ void pair_coef(const PairArgs& a, long long px, const float* tp, PairCoef<VEC>& q) {
+  float la[VEC], lo[VEC], lb[VEC], lt[VEC], gp[VEC], gk[VEC], mk[VEC], u0[VEC];
+  Vec<VEC>::load_cached(a.lse_all + px, la);
+  Vec<VEC>::load_cached(a.bkg_gap + px, lo);  // lse_all - lse_old where the label is 0 (the forward's loss_px)
+  Vec<VEC>::load_cached(a.lse3 + a.plane + px, lb);
+  Vec<VEC>::load_cached(a.lse3 + 2 * a.plane + px, lt);
+  Vec<VEC>::load_cached(tp, u0);
+  if (a.ce_g_px != nullptr) Vec<VEC>::load_cached(a.ce_g_px + px, gp);
+  if (a.kd_g_px != nullptr) Vec<VEC>::load_cached(a.kd_g_px + px, gk);
+  if (a.mask != nullptr) Vec<VEC>::load_cached(a.mask + px, mk);
+  const long long* yp = a.y + px;
+#pragma unroll
+  for (int i = 0; i < VEC; ++i) {
+    long long tt = yp[i];
+    if (tt < a.old_cl) tt = 0;
+    const bool dead = (tt == a.ignore_index) || tt < 0 || tt >= a.C;
+    q.lab[i] = dead ? -1 : (int)tt;
+    q.uce[i] = dead ? 0.f : (a.ce_g_px != nullptr ? gp[i] : a.gs_ce);
+    q.la2[i] = la[i] * kLog2e;
+    q.lt2[i] = lt[i] * kLog2e;
+    q.fold[i] = ex2f(lo[i] * kLog2e);
+    float u = (a.kd_g_px != nullptr ? gk[i] : a.gs_kd) * a.inv_cold;
+    if (a.mask != nullptr) u *= a.mask_zero ? (mk[i] == 0.f ? 1.f : 0.f) : mk[i];
+    q.ukd[i] = u;
+    const float q0 = ex2f(fmaf(u0[i], a.a2, -q.lt2[i]));
+    q.fb[i] = q0 * ex2f((la[i] - lb[i]) * kLog2e);
+  }
+}
+
+// dx of channel c at pixel i: v = x_c, u = t_c (read only for an old foreground class, 1 <= c < C_old)
+template <int VEC>
+__device__ __forceinline__ float pair_dx(const PairArgs& a, const PairCoef<VEC>& q, int i, int c, bool old_fg, float v,
+                                         float u) {
+  const float pr = ex2f(fmaf(v, kLog2e, -q.la2[i]));
+  float sub_ce;
+  if (q.lab[i] == 0 && a.old_cl > 0)
+    sub_ce = (c < a.old_cl) ? pr * q.fold[i] : 0.f;
+  else
+    sub_ce = (c == q.lab[i]) ? 1.f : 0.f;
+  const float sub_kd = old_fg ? ex2f(fmaf(u, a.a2, -q.lt2[i])) : pr * q.fb[i];
+  return fmaf(q.uce[i], pr - sub_ce, q.ukd[i] * (pr - sub_kd));
+}
+
 template <int VEC, bool ACC>
 __global__ void __launch_bounds__(kStreamThreads)
 unce_unkd_bwd_kernel(const float* __restrict__ x, const long long* __restrict__ y, const float* __restrict__ lse_all,
@@ -546,51 +632,17 @@ unce_unkd_bwd_kernel(const float* __restrict__ x, const long long* __restrict__ 
                      int mask_zero, float* __restrict__ dx, int B, int C, int C_old, long long HW) {
   const long long gpi = HW / VEC;
   const long long n_groups = gpi * B;
-  const long long plane = (long long)B * HW;
-  const float a2 = alpha * kLog2e;
-  const float inv_cold = 1.f / (float)C_old;
-  float gs_ce = 0.f;
-  if (ce_g_px == nullptr) {
-    gs_ce = ce_g_scalar[0] * ce_g_mul;
-    if (mean_over_valid) gs_ce = gs_ce / ce_stats[1];
-  }
-  const float gs_kd = (kd_g_px == nullptr) ? kd_g_scalar[0] * kd_g_mul : 0.f;
+  const PairArgs a = pair_args(y, lse_all, bkg_gap, ce_g_px, ce_g_scalar, ce_g_mul, ce_stats, mean_over_valid, old_cl,
+                               ignore_index, t, mask, alpha, lse3, kd_g_px, kd_g_scalar, kd_g_mul, mask_zero, B, C,
+                               C_old, HW);
   for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < n_groups;
        g += (long long)gridDim.x * blockDim.x) {
     const long long b = g / gpi, p = (g - b * gpi) * VEC;
     const float* xp = x + (b * C) * HW + p;
     const float* tp = t + (b * C_old) * HW + p;
     float* dp = dx + (b * C) * HW + p;
-    const long long* yp = y + b * HW + p;
-    float la2[VEC], lt2[VEC], uce[VEC], ukd[VEC], fold[VEC], fb[VEC];
-    int lab[VEC];
-    {
-      float la[VEC], lo[VEC], lb[VEC], lt[VEC], gp[VEC], gk[VEC], mk[VEC], u0[VEC];
-      Vec<VEC>::load_cached(lse_all + b * HW + p, la);
-      Vec<VEC>::load_cached(bkg_gap + b * HW + p, lo);  // lse_all - lse_old where the label is 0 (the forward's loss_px)
-      Vec<VEC>::load_cached(lse3 + plane + b * HW + p, lb);
-      Vec<VEC>::load_cached(lse3 + 2 * plane + b * HW + p, lt);
-      Vec<VEC>::load_cached(tp, u0);
-      if (ce_g_px != nullptr) Vec<VEC>::load_cached(ce_g_px + b * HW + p, gp);
-      if (kd_g_px != nullptr) Vec<VEC>::load_cached(kd_g_px + b * HW + p, gk);
-      if (mask != nullptr) Vec<VEC>::load_cached(mask + b * HW + p, mk);
-#pragma unroll
-      for (int i = 0; i < VEC; ++i) {
-        long long tt = yp[i];
-        if (tt < old_cl) tt = 0;
-        const bool dead = (tt == ignore_index) || tt < 0 || tt >= C;
-        lab[i] = dead ? -1 : (int)tt;
-        uce[i] = dead ? 0.f : (ce_g_px != nullptr ? gp[i] : gs_ce);
-        la2[i] = la[i] * kLog2e;
-        lt2[i] = lt[i] * kLog2e;
-        fold[i] = ex2f(lo[i] * kLog2e);
-        float u = (kd_g_px != nullptr ? gk[i] : gs_kd) * inv_cold;
-        if (mask != nullptr) u *= mask_zero ? (mk[i] == 0.f ? 1.f : 0.f) : mk[i];
-        ukd[i] = u;
-        const float q0 = ex2f(fmaf(u0[i], a2, -lt2[i]));
-        fb[i] = q0 * ex2f((la[i] - lb[i]) * kLog2e);
-      }
-    }
+    PairCoef<VEC> q;
+    pair_coef<VEC>(a, b * HW + p, tp, q);
 #pragma unroll 4
     for (int c = 0; c < C; ++c) {
       float v[VEC], u[VEC], o[VEC];
@@ -598,17 +650,142 @@ unce_unkd_bwd_kernel(const float* __restrict__ x, const long long* __restrict__ 
       const bool old_fg = c >= 1 && c < C_old;  // an old foreground class: KD subtracts q_c (uniform over the block)
       if (old_fg) Vec<VEC>::load(tp + (long long)c * HW, u);
 #pragma unroll
-      for (int i = 0; i < VEC; ++i) {
-        const float pr = ex2f(fmaf(v[i], kLog2e, -la2[i]));
-        float sub_ce;
-        if (lab[i] == 0 && old_cl > 0)
-          sub_ce = (c < old_cl) ? pr * fold[i] : 0.f;
-        else
-          sub_ce = (c == lab[i]) ? 1.f : 0.f;
-        const float sub_kd = old_fg ? ex2f(fmaf(u[i], a2, -lt2[i])) : pr * fb[i];
-        o[i] = fmaf(uce[i], pr - sub_ce, ukd[i] * (pr - sub_kd));
-      }
+      for (int i = 0; i < VEC; ++i) o[i] = pair_dx<VEC>(a, q, i, c, old_fg, v[i], u[i]);
       store_dx<VEC, ACC>(dp + (long long)c * HW, o);
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// The same backward contracted with the bilinear adjoint on the fly: d_lr = U^T dx with U the upsample of the logits
+// (sweep form, sweep_adjoint.cuh: integer scales, a multiple of 8 along x).  dx is formed in registers and never
+// written: the pass reads x, t, the labels and the saved planes once (4 C + 4 C_old + 24 B per pixel) and writes only
+// the low-res gradient.
+// block = (image b, range of low-res rows [y0, ylast], group of at most KMAX channels), the channel group fastest in the
+// grid so that the per-pixel planes, read by every group, come from L2 after the first.  thread = 4 consecutive X of
+// a full-res row (blockDim = W / 4), sweeping the full-res rows of the range top-down; per row and channel 8 FMAs fold
+// x and 4 fold y into 4 accumulators: (upper, lower) y tap x (upper, lower) x tap.  When the sweep leaves interval k
+// (the rows whose upper tap is k), low-res row k is emitted (shared-memory gather over the threads whose x taps hit
+// each cell, fixed order) and the lower-tap sums become the next interval's starting value.  The lower-tap sums of a
+// range's last interval belong to the next range's first row: that row receives exactly two contributions, its owner's
+// and this carry, added with atomicAdd onto a zeroed output (two operands commute: deterministic).
+// ------------------------------------------------------------------------------------------
+// KMAX: channels per block (a multiple of 4); NREG: register cap per thread (blocks of <= 256 threads)
+template <int KMAX, int NREG>
+__global__ void __maxnreg__(NREG)
+unce_unkd_bwd_lowres_kernel(const float* __restrict__ x, const long long* __restrict__ y,
+                            const float* __restrict__ lse_all, const float* __restrict__ bkg_gap,
+                            const float* __restrict__ ce_g_px, const float* __restrict__ ce_g_scalar, float ce_g_mul,
+                            const float* __restrict__ ce_stats, int mean_over_valid, int old_cl, int ignore_index,
+                            const float* __restrict__ t, const float* __restrict__ mask, float alpha,
+                            const float* __restrict__ lse3, const float* __restrict__ kd_g_px,
+                            const float* __restrict__ kd_g_scalar, float kd_g_mul, int mask_zero,
+                            float* __restrict__ d_lr, int B, int C, int C_old, int h, int w, int H, int W,
+                            float scale_h, float scale_w, int n_ranges, int range_rows, int n_cgroups, int ny_cap) {
+  extern __shared__ __align__(16) uint8_t lr_dyn[];
+  const int wv = blockDim.x;  // == W / 4
+  const int tid = threadIdx.x;
+  // 8-byte entries first: every array starts aligned whatever ny_cap and wv are
+  float2* s_p = reinterpret_cast<float2*>(lr_dyn);                 // [2][KMAX][wv] (p0, p1) of the rows being emitted
+  short4* s_j = reinterpret_cast<short4*>(s_p + 2 * KMAX * wv);    // [w] thread ranges hitting low-res x
+  float2* s_h = reinterpret_cast<float2*>(s_j + w);                // [ny_cap] y weights (upper tap, lower tap)
+  int* s_k = reinterpret_cast<int*>(s_h + ny_cap);                 // [ny_cap] low-res row of the upper tap
+  int* s_x0 = s_k + ny_cap;                                        // [wv] upper / lower x tap of each thread
+  int* s_x1 = s_x0 + wv;
+  __shared__ int s_lim[2];
+  const long long HW = (long long)H * W;
+  const PairArgs a = pair_args(y, lse_all, bkg_gap, ce_g_px, ce_g_scalar, ce_g_mul, ce_stats, mean_over_valid, old_cl,
+                               ignore_index, t, mask, alpha, lse3, kd_g_px, kd_g_scalar, kd_g_mul, mask_zero, B, C,
+                               C_old, HW);
+  const int cg = blockIdx.x % n_cgroups;
+  const int rest = blockIdx.x / n_cgroups;
+  const int rg = rest % n_ranges;
+  const long long b = rest / n_ranges;
+  const int c0 = (int)((long long)cg * C / n_cgroups), kc = (int)((long long)(cg + 1) * C / n_cgroups) - c0;
+  const int y0 = rg * range_rows, ylast = min(h, y0 + range_rows) - 1;
+  float wx0[4], wx1[4];
+  sweep_x_taps(tid, wv, w, W, scale_w, wx0, wx1, s_x0, s_x1, s_j);
+  int i_lo, i_hi;
+  const int Ylo = sweep_y_taps(tid, wv, y0, ylast, h, H, scale_h, ny_cap, s_k, s_h, s_lim, i_lo, i_hi);
+  const int X = tid * 4;
+  const float* xb = x + (b * C + c0) * HW + X;
+  const float* tb = t + b * C_old * HW + X;
+  float* out = d_lr + (b * C + c0) * (long long)h * w;
+  // accumulators per channel: a0 = towards low-res row `cur` (upper y tap), a1 = towards row cur + 1 (lower y tap);
+  // .x / .y = upper / lower x tap
+  float2 a0[KMAX], a1[KMAX];
+#pragma unroll
+  for (int j = 0; j < KMAX; ++j) a0[j] = a1[j] = make_float2(0.f, 0.f);
+  int cur = -1, flip = 0;
+  // low-res row `row` of the block's channels += gather over x of the per-thread pairs in a0; `shared`: another block
+  // contributes to this row as well
+  auto emit = [&](int row, bool shared) {
+    float2* sp = s_p + flip * KMAX * wv;
+#pragma unroll
+    for (int j = 0; j < KMAX; ++j)
+      if (j < kc) sp[j * wv + tid] = a0[j];
+    __syncthreads();  // one barrier per emit: the buffers alternate, so the next emit cannot overtake this gather
+    for (int o = tid; o < kc * w; o += wv) {
+      const int j = o / w, xo = o - j * w;
+      const short4 jr = s_j[xo];
+      const float2* pj = sp + j * wv;
+      float acc = 0.f;
+      for (int i = jr.x; i < jr.y; ++i) acc += pj[i].x;
+      for (int i = jr.z; i < jr.w; ++i) acc += pj[i].y;
+      float* dst = out + ((long long)j * h + row) * w + xo;
+      if (shared)
+        atomicAdd(dst, acc);
+      else
+        *dst = acc;
+    }
+    flip ^= 1;
+  };
+#pragma unroll 1
+  for (int i = i_lo; i < i_hi; ++i) {
+    const int k = s_k[i];
+    if (k != cur) {  // uniform over the block
+      if (cur >= 0) {
+        emit(cur, cur == y0 && y0 > 0);
+#pragma unroll
+        for (int j = 0; j < KMAX; ++j) a0[j] = a1[j], a1[j] = make_float2(0.f, 0.f);
+      }
+      cur = k;
+    }
+    const long long row = (long long)(Ylo + i) * W;
+    PairCoef<4> q;
+    pair_coef<4>(a, b * HW + row + X, tb + row, q);
+    const float2 hw = s_h[i];
+#pragma unroll
+    for (int j0 = 0; j0 < KMAX; j0 += 4) {  // 4 channels of x and t in flight, then their arithmetic
+      float v[4][4], u[4][4];
+#pragma unroll
+      for (int jj = 0; jj < 4; ++jj) {
+        const int c = c0 + j0 + jj;
+        if (j0 + jj < kc) Vec<4>::load(xb + (long long)(j0 + jj) * HW + row, v[jj]);
+        if (j0 + jj < kc && c >= 1 && c < C_old) Vec<4>::load(tb + (long long)c * HW + row, u[jj]);
+      }
+#pragma unroll
+      for (int jj = 0; jj < 4; ++jj) {
+        const int j = j0 + jj, c = c0 + j;
+        if (j < kc) {
+          const bool old_fg = c >= 1 && c < C_old;
+          float o[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) o[e] = pair_dx<4>(a, q, e, c, old_fg, v[jj][e], u[jj][e]);
+          const float p0 = fmaf(o[3], wx0[3], fmaf(o[2], wx0[2], fmaf(o[1], wx0[1], o[0] * wx0[0])));
+          const float p1 = fmaf(o[3], wx1[3], fmaf(o[2], wx1[2], fmaf(o[1], wx1[1], o[0] * wx1[0])));
+          a0[j].x = fmaf(hw.x, p0, a0[j].x), a0[j].y = fmaf(hw.x, p1, a0[j].y);
+          a1[j].x = fmaf(hw.y, p0, a1[j].x), a1[j].y = fmaf(hw.y, p1, a1[j].y);
+        }
+      }
+    }
+  }
+  if (cur >= 0) {
+    emit(cur, cur == y0 && y0 > 0);
+    if (ylast < h - 1) {  // lower-tap sums of the last interval: the next range's first row
+#pragma unroll
+      for (int j = 0; j < KMAX; ++j) a0[j] = a1[j];
+      emit(ylast + 1, true);
     }
   }
 }
@@ -792,5 +969,93 @@ extern "C" int ucd_unce_unkd_bwd(const float* x, const int64_t* y, const float* 
                                         ce_stats, mean_over_valid, old_cl, ignore_index, t, mask, alpha, lse3, kd_g_px,
                                         kd_g_scalar, kd_g_mul, kd_variant == 2 ? 1 : 0, dx, B, C, C_old, HW);
   UCD_CHECK_LAUNCH("unce_unkd_bwd_kernel");
+  return UCD_OK;
+}
+
+extern "C" int ucd_unce_unkd_bwd_lowres(const float* x, const int64_t* y, const float* lse_all, const float* bkg_gap,
+                                        const float* ce_g_px, const float* ce_g_scalar, float ce_g_mul,
+                                        const float* ce_stats, int mean_over_valid, int old_cl, int ignore_index,
+                                        const float* t, const float* mask, float alpha, const float* lse3,
+                                        const float* kd_g_px, const float* kd_g_scalar, float kd_g_mul, int kd_variant,
+                                        float* d_lr, int B, int C, int C_old, int h, int w, int H, int W,
+                                        void* stream) {
+  UCD_CHECK_ARG(x && y && lse_all && bkg_gap && t && lse3 && d_lr, "ucd_unce_unkd_bwd_lowres: null pointer");
+  UCD_CHECK_ARG((ce_g_px || ce_g_scalar) && (kd_g_px || kd_g_scalar),
+                "ucd_unce_unkd_bwd_lowres: need g_px or g_scalar for both terms");
+  UCD_CHECK_ARG(!mean_over_valid || ce_stats, "ucd_unce_unkd_bwd_lowres: mean_over_valid needs stats");
+  UCD_CHECK_ARG(B > 0 && C_old >= 1 && C >= C_old && h > 0 && w > 0 && H > 0 && W > 0,
+                "ucd_unce_unkd_bwd_lowres: bad shape");
+  UCD_CHECK_ARG(kd_variant == 0 || kd_variant == 2,
+                "ucd_unce_unkd_bwd_lowres: KD variant must be 0 (unbiased) or 2 (masked)");
+  // the sweep form of the adjoint (sweep_adjoint.cuh): integer scales, a multiple of 8 along x, one block row = W/4
+  // threads; everything else is the caller's two-step path (ucd_unce_unkd_bwd + ucd_upsample_bilinear_bwd)
+  const int up = H / h;
+  const bool ok = H % h == 0 && W % w == 0 && (W / w) % 8 == 0 && W / 4 <= 256 && (W / 4) % 32 == 0 && w <= W / 4 &&
+                  can_vec4((long long)H * W, {x, lse_all, bkg_gap, ce_g_px, t, mask, lse3, kd_g_px}) && aligned16(y) &&
+                  up <= 64;
+  if (!ok) {
+    set_error("ucd_unce_unkd_bwd_lowres: %dx%d -> %dx%d is not a sweep-form shape", h, w, H, W);
+    return UCD_ENOSUP;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int wv = W / 4;
+  struct Variant {
+    int k, nreg;
+    void (*fn)(const float*, const long long*, const float*, const float*, const float*, const float*, float,
+               const float*, int, int, int, const float*, const float*, float, const float*, const float*,
+               const float*, float, int, float*, int, int, int, int, int, int, int, float, float, int, int, int, int);
+  };
+  static const Variant variants[] = {{8, 128, unce_unkd_bwd_lowres_kernel<8, 128>},
+                                     {4, 128, unce_unkd_bwd_lowres_kernel<4, 128>},
+#ifdef UCD_DEBUG_KNOBS  // tighter register caps: more warps per SM, a few spilled registers
+                                     {4, 96, unce_unkd_bwd_lowres_kernel<4, 96>},
+                                     {8, 112, unce_unkd_bwd_lowres_kernel<8, 112>},
+#endif
+  };
+  int vi = 0;
+#ifdef UCD_DEBUG_KNOBS
+  if (const char* e = getenv("UCD_LRB_VARIANT")) vi = (atoi(e) >= 0 && atoi(e) < 4) ? atoi(e) : 0;  // tuning knob
+#endif
+  const Variant& var = variants[vi];
+  // Grid: enough threads for ~2 waves of what the registers let reside per SM.  Fewer low-res rows per range first
+  // (each range boundary costs one extra row emit), then more, smaller channel groups (each group re-reads the
+  // per-pixel planes from L2 and recomputes the coefficients).
+  const int min_groups = (C + var.k - 1) / var.k;
+  int groups = min_groups, rows = h;
+  const long long want = 2ll * kNumSMs * (65536 / var.nreg / 32 * 32);
+  auto threads = [&](int r, int g) { return (long long)B * ((h + r - 1) / r) * g * wv; };
+  while (rows > 1 && threads(rows, groups) < want) rows = (rows + 1) / 2;
+  while (groups < C && threads(rows, groups) < want) ++groups;
+  // the tap table of one range must fit in shared memory
+  auto dyn_bytes = [&](int r) {
+    return (size_t)2 * var.k * wv * 8 + (size_t)w * 8 + (size_t)((r + 2) * up + 8) * 12 + (size_t)2 * wv * 4;
+  };
+#ifdef UCD_DEBUG_KNOBS
+  if (const char* e = getenv("UCD_LRB_ROWS")) rows = atoi(e) > 0 ? min(atoi(e), h) : rows;  // tuning knobs
+  if (const char* e = getenv("UCD_LRB_GROUPS")) groups = atoi(e) >= min_groups ? min(atoi(e), C) : groups;
+#endif
+  while (rows > 1 && dyn_bytes(rows) > 200 * 1024) rows = (rows + 1) / 2;
+  const int n_ranges = (h + rows - 1) / rows;
+  const long long nb = (long long)B * n_ranges * groups;
+  if (nb >= (1ll << 31) || dyn_bytes(rows) > 200 * 1024) {
+    set_error("ucd_unce_unkd_bwd_lowres: B=%d h=%d H=%d needs more blocks or shared memory than one launch has", B, h, H);
+    return UCD_ENOSUP;
+  }
+  const int ny_cap = (rows + 2) * up + 8;
+  const size_t dyn = dyn_bytes(rows);
+  auto kern = var.fn;
+  cudaError_t e;
+  if (dyn > 48 * 1024) {
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(unce_unkd_bwd_lowres)");
+  }
+  // range boundary rows receive two contributions (see the kernel): the output starts from zero
+  e = cudaMemsetAsync(d_lr, 0, (size_t)B * C * h * w * sizeof(float), st);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(unce_unkd_bwd_lowres)");
+  kern<<<(unsigned)nb, wv, dyn, st>>>(x, (const long long*)y, lse_all, bkg_gap, ce_g_px, ce_g_scalar, ce_g_mul,
+                                      ce_stats, mean_over_valid, old_cl, ignore_index, t, mask, alpha, lse3, kd_g_px,
+                                      kd_g_scalar, kd_g_mul, kd_variant == 2 ? 1 : 0, d_lr, B, C, C_old, h, w, H, W,
+                                      (float)h / (float)H, (float)w / (float)W, n_ranges, rows, groups, ny_cap);
+  UCD_CHECK_LAUNCH("unce_unkd_bwd_lowres_kernel");
   return UCD_OK;
 }

@@ -9,6 +9,7 @@
 // plane, streams the full-res rows that touch them once (coalesced), reduces them along y in
 // registers, then along x out of shared memory.  No atomics; summation order is fixed.
 #include "common.cuh"
+#include "sweep_adjoint.cuh"
 
 #include <stdlib.h>
 
@@ -301,43 +302,17 @@ upsample_bwd_sweep_kernel(const float* __restrict__ gout, float* __restrict__ gi
   const int wv = blockDim.x;  // == W / 4
   const int tid = threadIdx.x;
   float4* ring = reinterpret_cast<float4*>(up_dyn);                       // [UN][wv]
+  // 8-byte entries first: every array starts aligned whatever ny_cap and wv are
   float2* s_p = reinterpret_cast<float2*>(ring + (size_t)UN * wv);        // [2][wv] (p0, p1) of the row being emitted
-  float2* s_h = s_p + 2 * wv;                                             // [ny_cap] y weights (upper tap, lower tap)
+  short4* s_j = reinterpret_cast<short4*>(s_p + 2 * wv);                  // [w] thread ranges hitting low-res x
+  float2* s_h = reinterpret_cast<float2*>(s_j + w);                       // [ny_cap] y weights (upper tap, lower tap)
   int* s_k = reinterpret_cast<int*>(s_h + ny_cap);                        // [ny_cap] low-res row of the upper tap
   int* s_x0 = s_k + ny_cap;                                               // [wv] upper / lower x tap of each thread
   int* s_x1 = s_x0 + wv;
-  short4* s_j = reinterpret_cast<short4*>(s_x1 + wv);                     // [w] thread ranges hitting low-res x
   __shared__ int s_lim[2];                                                // first / last+1 tap-table row actually read
   const int X = tid * 4;
   float wx0[4], wx1[4];
-  {
-    const Tap t0 = bilinear_tap(X, scale_w, w, W);
-    s_x0[tid] = t0.i0, s_x1[tid] = t0.i1;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const Tap tx = bilinear_tap(X + i, scale_w, w, W);  // same i0 / i1 as t0 (host-checked precondition)
-      wx0[i] = tx.w0, wx1[i] = tx.w1;
-    }
-  }
-  __syncthreads();
-  if (tid < w) {  // thread ranges per low-res column (taps are monotone in X, so the hits are contiguous)
-    const int sc4 = (W / w) / 4;
-    const int j0 = max((tid - 2) * sc4 - 2, 0), j1 = min((tid + 2) * sc4 + 2, wv - 1);
-    int a0 = 0, a1 = 0, b0 = 0, b1 = 0;
-    bool fa = false, fb = false;
-    for (int j = j0; j <= j1; ++j) {
-      if (s_x0[j] == tid) {
-        if (!fa) a0 = j, fa = true;
-        a1 = j + 1;
-      }
-      if (s_x1[j] == tid) {
-        if (!fb) b0 = j, fb = true;
-        b1 = j + 1;
-      }
-    }
-    s_j[tid] = make_short4((short)a0, (short)a1, (short)b0, (short)b1);
-  }
-  const float inv = (float)H / (float)h;
+  sweep_x_taps(tid, wv, w, W, scale_w, wx0, wx1, s_x0, s_x1, s_j);
   const uint32_t ring_s = (uint32_t)__cvta_generic_to_shared(ring + tid);  // this thread's 16 B of slot 0
   const uint32_t slot_b = (uint32_t)wv * 16u;
   int flip = 0;
@@ -349,28 +324,8 @@ upsample_bwd_sweep_kernel(const float* __restrict__ gout, float* __restrict__ gi
     const int y0 = (int)(r - plane * h);
     const int ylast = (int)min((long long)min(h, y0 + cap_rows), y0 + (r_end - r)) - 1;
     r += ylast - y0 + 1;
-    int Ylo = (int)floorf(((float)y0 - 0.5f) * inv) - 2, Yhi = (int)ceilf(((float)ylast + 1.5f) * inv) + 2;
-    Ylo = max(Ylo, 0), Yhi = min(Yhi, H - 1);
-    const int ny = min(Yhi - Ylo + 1, ny_cap);
-    __syncthreads();  // the previous segment no longer reads the tap table
-    for (int i = tid; i < ny; i += wv) {
-      const Tap ty = bilinear_tap(Ylo + i, scale_h, h, H);
-      s_k[i] = ty.i0;
-      const bool clamped = ty.i1 == ty.i0;  // bottom border: both taps hit the same low-res row
-      s_h[i] = make_float2(clamped ? ty.w0 + ty.w1 : ty.w0, clamped ? 0.f : ty.w1);
-    }
-    __syncthreads();
-    // rows whose upper tap lies in [y0, ylast] are the ones to read (the rest are margins of the conservative range);
-    // s_k is monotone, so exactly one row starts and one row ends that run
-    for (int i = tid; i < ny; i += wv) {
-      const int k = s_k[i];
-      if (k >= y0 && k <= ylast) {
-        if (i == 0 || s_k[i - 1] < y0) s_lim[0] = i;
-        if (i == ny - 1 || s_k[i + 1] > ylast) s_lim[1] = i + 1;
-      }
-    }
-    __syncthreads();
-    const int i_lo = s_lim[0], i_hi = s_lim[1];
+    int i_lo, i_hi;
+    const int Ylo = sweep_y_taps(tid, wv, y0, ylast, h, H, scale_h, ny_cap, s_k, s_h, s_lim, i_lo, i_hi);
     const float* gp = gout + (size_t)plane * H * W + (size_t)(Ylo + i_lo) * W + X;  // next row to fetch
     float* out = gin + (size_t)plane * h * w;
     float a0p0 = 0.f, a0p1 = 0.f, a1p0 = 0.f, a1p1 = 0.f, c0 = 0.f, c1 = 0.f;  // current interval, carry from the one above

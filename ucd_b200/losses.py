@@ -21,6 +21,8 @@ There is no CPU path: CPU tensors or a missing library raise.
 """
 from __future__ import annotations
 
+import weakref
+
 import torch
 import torch.nn as nn
 
@@ -70,6 +72,7 @@ class _UpsampleFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, out_h, out_w):
         _need_cuda(x)
+        ctx.set_materialize_grads(False)   # no gradient reaches `out` when a loss chain hands d x straight to x (_Route)
         x = _f32c(x)
         lead, (h, w) = x.shape[:-2], x.shape[-2:]
         planes = 1
@@ -84,6 +87,8 @@ class _UpsampleFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        if g is None:
+            return None, None, None
         lead, h, w, out_h, out_w, planes = ctx.shape
         g = _f32c(g)
         gin = torch.empty(*lead, h, w, device=g.device, dtype=torch.float32)
@@ -95,7 +100,58 @@ class _UpsampleFn(torch.autograd.Function):
 
 def interpolate_bilinear(x, size):
     """``F.interpolate(x, size=size, mode='bilinear', align_corners=False)`` (segmentation_module.py:133)."""
-    return _UpsampleFn.apply(x, int(size[0]), int(size[1]))
+    out = _UpsampleFn.apply(x, int(size[0]), int(size[1]))
+    if out.requires_grad:   # where `out` came from, for a loss chain that folds the adjoint into its backward (_Route)
+        out._ucd_upsample = (x, x._version, out._version)
+    return out
+
+
+class _Route:
+    """Lets the head of a gradient chain on `outputs` = interpolate_bilinear(lr) hand the gradient of the LOW-RES logits
+    straight to `lr` (``ucd_unce_unkd_bwd_lowres``: the full-size dx is never written, nor read back by the adjoint),
+    instead of dx to `outputs`.  The head's Function then takes `lr` as an extra autograd input; `outputs`' own node
+    receives no gradient from the chain (other consumers of `outputs` still flow through it and add up at `lr`).
+
+    That is only equivalent while nobody observes the gradient of `outputs` itself.  `route_now()` decides in the
+    head's backward, and anything it cannot classify takes the old path (dx for `outputs`):
+      * `outputs.retains_grad` or tensor hooks on `outputs`: old path;
+      * the pass must be a plain ``backward()``: ``autograd.grad`` / ``backward(inputs=...)`` may capture the gradient of
+        `outputs`, and the engine cannot say whether it does (a captured node reads as "will execute").  A private leaf
+        (`probe`) that no caller can name is an extra input of the head: its node executes in a plain pass only.
+    Not covered: hooks registered on the NODE of `outputs` (``outputs.grad_fn.register_prehook`` / ``register_hook``)
+    receive no gradient from the chain when it reroutes - torch offers no way to see them.  A tensor hook
+    (``outputs.register_hook``) observes the same gradient and keeps the old path."""
+
+    __slots__ = ("lr_shape", "out_ref", "out_hw", "probe_node")
+    _probes = {}
+
+    def __init__(self, src, out, probe_node):
+        self.lr_shape, self.out_hw, self.probe_node = tuple(src.shape), tuple(out.shape[2:]), probe_node
+        self.out_ref = weakref.ref(out)
+
+    @staticmethod
+    def of(outputs):
+        """(route, lr, probe) when `outputs` is still what interpolate_bilinear(lr) returned, else None."""
+        rec = getattr(outputs, "_ucd_upsample", None)
+        if rec is None:
+            return None
+        src, src_version, out_version = rec
+        if (src._version != src_version or outputs._version != out_version or not src.requires_grad
+                or src.dim() != 4 or outputs.dim() != 4):
+            return None
+        probe = _Route._probes.get(outputs.device)
+        if probe is None:
+            probe = _Route._probes[outputs.device] = torch.empty((), device=outputs.device, requires_grad=True)
+        return _Route(src, outputs, torch.autograd.graph.get_gradient_edge(probe).node), src, probe
+
+    def route_now(self):
+        out = self.out_ref()
+        if out is None or out.retains_grad or out._backward_hooks:
+            return False
+        try:
+            return bool(torch._C._will_engine_execute_node(self.probe_node))
+        except Exception:   # noqa: BLE001 - e.g. a torch that no longer offers it: the old path is always right
+            return False
 
 
 # ----------------------------------------------------------------------------------------------
@@ -134,28 +190,64 @@ class _GradChain:
             chain = t._ucd_grad_chain = _GradChain()
         return chain
 
-    def submit(self, term, seq, is_head):
-        """Called from a member's backward: returns (gradient for `inputs`, gradient for the link token)."""
+    def submit(self, term, seq, is_head, route=None):
+        """Called from a member's backward: returns (gradient for `inputs`, gradient for the link token, gradient for
+        the head's low-res source, see _Route)."""
         self.closed = True
         if seq == self.calls:      # the last call runs first in a backward pass: drop what a pass that died left behind
             self.pending = []
         if not is_head:
             if term is not None:
                 self.pending.append(term)
-            return None, None   # the token's gradient stays undefined: the edge alone orders the backward passes
+            return None, None, None   # the token's gradient stays undefined: the edge alone orders the backward passes
         terms, self.pending = self.pending + ([term] if term is not None else []), []
         self.token = None   # chain -> token -> grad_fn -> ctx -> chain would leave the pass's objects to the cycle collector
-        return (_launch_terms(terms) if terms else None), None
+        if not terms:
+            return None, None, None
+        d_lr = _launch_lowres(terms, route) if route is not None else None
+        if d_lr is not None:
+            return None, None, d_lr
+        return _launch_terms(terms), None, None
+
+
+def _pair(terms):
+    """(ce term, kd term) that one kernel can run together, or None."""
+    ce = [t for t in terms if t["kind"] == "ce"]
+    kd = [t for t in terms if t["kind"] == "kd" and t["variant"] in (0, 2)]
+    if ce and kd and ce[0]["C"] == kd[0]["C"] and ce[0]["HW"] == kd[0]["HW"]:
+        return ce[0], kd[0]
+    return None
+
+
+def _launch_lowres(terms, route):
+    """d lr for a chain of exactly a cross-entropy + distillation pair, with the upsample adjoint folded in; None when
+    the pass may observe the gradient of `outputs` or the shape is not one the kernel takes (the caller then runs the
+    old path)."""
+    pair = _pair(terms)
+    if pair is None or len(terms) != 2 or not route.route_now():
+        return None
+    c, k = pair
+    B, C, h, w = route.lr_shape
+    H, W = route.out_hw
+    d_lr = torch.empty(B, C, h, w, device=c["x"].device, dtype=torch.float32)
+    rc = _lib.lib().ucd_unce_unkd_bwd_lowres(
+        ptr(c["x"]), ptr(c["targets"]), ptr(c["lse"][0]), ptr(c["lse"][1]), ptr(c["g_px"]), ptr(c["g_sc"]), 1.0,
+        ptr(c["stats"]), c["mean_over_valid"], c["old_cl"], c["ignore_index"], ptr(k["t"]), ptr(k["m"]), k["alpha"],
+        ptr(k["lse3"]), ptr(k["g_px"]), ptr(k["g_sc"]), k["g_mul"], k["variant"], ptr(d_lr), B, C, k["C_old"], h, w,
+        H, W, cur_stream())
+    if rc == _lib.UCD_ENOSUP:
+        return None
+    check(rc, "unce_unkd_bwd_lowres")
+    return d_lr
 
 
 def _launch_terms(terms):
     """dx = sum of the terms' logit gradients, written by as few passes over the logits as possible."""
     dx = torch.empty_like(terms[0]["x"])
-    ce = [t for t in terms if t["kind"] == "ce"]
-    kd = [t for t in terms if t["kind"] == "kd" and t["variant"] in (0, 2)]
+    pair = _pair(terms)
     acc = False
-    if ce and kd and ce[0]["C"] == kd[0]["C"] and ce[0]["HW"] == kd[0]["HW"]:
-        c, k = ce[0], kd[0]
+    if pair is not None:
+        c, k = pair
         check(_lib.lib().ucd_unce_unkd_bwd(
             ptr(c["x"]), ptr(c["targets"]), ptr(c["lse"][0]), ptr(c["lse"][1]), ptr(c["g_px"]), ptr(c["g_sc"]), 1.0,
             ptr(c["stats"]), c["mean_over_valid"], c["old_cl"], c["ignore_index"], ptr(k["t"]), ptr(k["m"]), k["alpha"],
@@ -186,8 +278,10 @@ def _launch_term(t, dx, acc):
 # ----------------------------------------------------------------------------------------------
 class _UnceFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, inputs, targets, old_cl, ignore_index, reduction, chain=None, link=None):
+    def forward(ctx, inputs, targets, old_cl, ignore_index, reduction, chain=None, link=None, route=None, src=None,
+                probe=None):
         ctx.chain, ctx.is_head, ctx.seq = chain, link is None, (chain.calls if chain is not None else 0)
+        ctx.route = route
         ctx.set_materialize_grads(False)   # the link token's gradient stays undefined: no zero tensors, no fill kernels
         B, C = inputs.shape[0], inputs.shape[1]
         HW = inputs.numel() // max(B * C, 1)
@@ -217,9 +311,9 @@ class _UnceFn(torch.autograd.Function):
         B, C, HW, old_cl, ignore_index, reduction = ctx.cfg
         if g is None:   # this loss value was not used: only the chain bookkeeping remains
             if ctx.chain is None:
-                return None, None, None, None, None, None, None
-            d_in, d_link = ctx.chain.submit(None, ctx.seq, ctx.is_head)
-            return d_in, None, None, None, None, None, d_link
+                return (None,) * 10
+            d_in, d_link, d_src = ctx.chain.submit(None, ctx.seq, ctx.is_head, ctx.route)
+            return d_in, None, None, None, None, None, d_link, None, d_src, None
         g_px, g_sc = None, None
         if reduction == "none":
             g_sc = _scalar_grad(g)
@@ -235,9 +329,9 @@ class _UnceFn(torch.autograd.Function):
         if ctx.chain is None:
             dx = torch.empty_like(x)
             _launch_term(term, dx, False)
-            return dx, None, None, None, None, None, None
-        d_in, d_link = ctx.chain.submit(term, ctx.seq, ctx.is_head)
-        return d_in, None, None, None, None, None, d_link
+            return (dx,) + (None,) * 9
+        d_in, d_link, d_src = ctx.chain.submit(term, ctx.seq, ctx.is_head, ctx.route)
+        return d_in, None, None, None, None, None, d_link, None, d_src, None
 
 
 def _chained(fn, inputs, args):
@@ -245,8 +339,14 @@ def _chained(fn, inputs, args):
     chain = _GradChain.of(inputs)
     if chain is None:
         return fn.apply(inputs, *args)
+    route = None
+    if chain.token is None:   # the head: it may hand the gradient to the low-res logits directly (_Route)
+        route = _Route.of(inputs)
     chain.calls += 1
-    out, token = fn.apply(inputs, *args, chain, chain.token)
+    if route is None:
+        out, token = fn.apply(inputs, *args, chain, chain.token)
+    else:
+        out, token = fn.apply(inputs, *args, chain, chain.token, *route)
     chain.token = token
     return out
 
@@ -282,8 +382,10 @@ class UnbiasedCrossEntropy(nn.Module):
 # ----------------------------------------------------------------------------------------------
 class _UnkdFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, inputs, targets, mask, alpha, reduction, variant=0, chain=None, link=None):
+    def forward(ctx, inputs, targets, mask, alpha, reduction, variant=0, chain=None, link=None, route=None, src=None,
+                probe=None):
         ctx.chain, ctx.is_head, ctx.seq = chain, link is None, (chain.calls if chain is not None else 0)
+        ctx.route = route
         ctx.set_materialize_grads(False)   # see _UnceFn
         B, C, C_old = inputs.shape[0], inputs.shape[1], targets.shape[1]
         HW = inputs.numel() // max(B * C, 1)
@@ -312,9 +414,9 @@ class _UnkdFn(torch.autograd.Function):
         B, C, C_old, HW, alpha, reduction, variant = ctx.cfg
         if g is None:   # this loss value was not used: only the chain bookkeeping remains
             if ctx.chain is None:
-                return None, None, None, None, None, None, None, None
-            d_in, d_link = ctx.chain.submit(None, ctx.seq, ctx.is_head)
-            return d_in, None, None, None, None, None, None, d_link
+                return (None,) * 11
+            d_in, d_link, d_src = ctx.chain.submit(None, ctx.seq, ctx.is_head, ctx.route)
+            return d_in, None, None, None, None, None, None, d_link, None, d_src, None
         g_px, g_sc, g_mul = None, None, 1.0
         if reduction == "none":
             g_sc = _scalar_grad(g)
@@ -331,9 +433,9 @@ class _UnkdFn(torch.autograd.Function):
         if ctx.chain is None:
             dx = torch.empty_like(x)
             _launch_term(term, dx, False)
-            return dx, None, None, None, None, None, None, None
-        d_in, d_link = ctx.chain.submit(term, ctx.seq, ctx.is_head)
-        return d_in, None, None, None, None, None, None, d_link
+            return (dx,) + (None,) * 10
+        d_in, d_link, d_src = ctx.chain.submit(term, ctx.seq, ctx.is_head, ctx.route)
+        return d_in, None, None, None, None, None, None, d_link, None, d_src, None
 
 
 class UnbiasedKnowledgeDistillationLoss(nn.Module):
