@@ -814,11 +814,15 @@ __global__ void __launch_bounds__(kConThreads, 1) con_sweep_kernel(const ConArgs
         proc(0, r0);
         proc(1, r1);
       } else {
-        // uniform tile: all 128 column labels equal this lane's row label, for every lane of the warp
+        // uniform tile: the 32 row labels of the warp are one label and all 128 column labels equal it.  Lane k
+        // compares only columns 4k..4k+3, so the row labels must be checked on their own: a warp with rows a|b split
+        // at lane K against a tile with columns a|b split at 4K passes the column compare alone.  Rows past n_rows
+        // (la = -2) never pass.
         bool uniform = false;
         if (PMODE != 2 && PMODE != 3 && full && !self) {
           const int4 l4 = *reinterpret_cast<const int4*>(lab + lane * 4);
-          uniform = __all_sync(0xffffffffu, l4.x == la && l4.y == la && l4.z == la && l4.w == la);
+          uniform = __all_sync(0xffffffffu, la == __shfl_sync(0xffffffffu, la, 0) && l4.x == la && l4.y == la &&
+                                                l4.z == la && l4.w == la);
         }
         const bool ones = PMODE == 0 || la >= thr;  // warp-uniform when `uniform` (same la, hence same thr, in every lane)
 #pragma unroll 1
