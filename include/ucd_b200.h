@@ -113,6 +113,11 @@ int ucd_upsample_bilinear_fwd(const float* in, float* out, int64_t planes, int h
                               void* stream);
 int ucd_upsample_bilinear_bwd(const float* gout, float* gin, int64_t planes, int h, int w, int H, int W,
                               void* stream);
+/* Prediction without the upsample: pred [B,H,W] int64 = argmax over the C channels of what
+ * ucd_upsample_bilinear_fwd writes for lr [B,C,h,w], bit for bit (same taps and operation order; ties go to the first
+ * maximal channel, NaN counts as maximal, as torch.argmax).  No [B,C,H,W] tensor is written or allocated.
+ * Upsampling only (H >= h, W >= w): downscaling returns UCD_EINVAL. */
+int ucd_upsample_argmax(const float* lr, int64_t* pred, int B, int C, int h, int w, int H, int W, void* stream);
 /* ucd_unce_unkd_bwd contracted with the adjoint of ucd_upsample_bilinear_fwd: when the logits x [B,C,H,W] are the
  * upsample of lr [B,C,h,w], d_lr [B,C,h,w] = upsample_adjoint(dx) of the dx ucd_unce_unkd_bwd would write (same
  * per-element values; the adjoint's summation order is its own).  dx is never written: one read-only pass over x, t,
@@ -134,6 +139,9 @@ int ucd_unce_unkd_bwd_lowres(const float* x, const int64_t* y, const float* lse_
  * with kd_px = -loss_px of the KD term, and (need_grad) the unit gradients g_ce, g_kd [B,C,h,w] of the two sums
  * with respect to lr.  Cross-block sums go through `workspace` (ucd_seg_fused_workspace_floats floats, 16 B
  * aligned) and are added in a fixed order: bit-identical from run to run.
+ * CE-only form (the base step, which has no old model): C_old == 0 with lr_old == NULL.  Only the CE is computed,
+ * g_kd is neither read nor written (may be NULL) and alpha is ignored; sums[2] = 0.  With old_cl == 0 the CE is plain
+ * cross-entropy (the background branch needs old_cl > 0).
  * ---------------------------------------------------------------------------------------- */
 size_t ucd_seg_fused_workspace_floats(int B, int C, int C_old, int h, int w, int H, int W);
 int ucd_seg_fused_fwd(const float* lr, const float* lr_old, int64_t* labels, float* g_ce, float* g_kd,

@@ -34,6 +34,7 @@ _PROTOS = {
     "ucd_bkg_mask": (c_int, [P, P, P, c_int, c_int, c_int64, c_int, P]),
     "ucd_upsample_bilinear_fwd": (c_int, [P, P, c_int64, c_int, c_int, c_int, c_int, P]),
     "ucd_upsample_bilinear_bwd": (c_int, [P, P, c_int64, c_int, c_int, c_int, c_int, P]),
+    "ucd_upsample_argmax": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ucd_seg_fused_workspace_floats": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int, c_int]),
     "ucd_seg_fused_fwd": (c_int, [P, P, P, P, P, P, P, c_size_t, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                   c_int, c_int, c_float, c_int, P]),

@@ -20,6 +20,8 @@
 //     rows with the y-tap weights into 4 values per (channel, column); four channels at a time these go to shared
 //     memory, and one thread per low-res cell folds the x-tap weights over the cell's (contiguous) column range and
 //     the row groups in a fixed order - 3x fewer instructions than a segmented shuffle reduction per channel.
+// CE-only form (KD = false, C_old = 0, no old model: the base step): phase A keeps the all-class and old-class
+// log-sum-exps only, phase B forms dCE only, and shared memory, the slabs and the gather carry one gradient term.
 // Cross-block sums (a low-res cell collects from <= 3 (interval, tap row) sources x <= 3 column tiles; the three loss
 // sums from every block) go through per-block slabs and a second kernel that adds them in a fixed order: like the
 // rest of the library the results are bit-identical from run to run (no atomics).
@@ -36,8 +38,8 @@ struct FusedArgs {
   const float* lo;      // [B,C_old,h,w]
   long long* labels;    // [B,H,W] (remapped in place like UnbiasedCrossEntropy)
   float* g_ce;          // [B,C,h,w]  d(sum_px ce_px)/d lr
-  float* g_kd;          // [B,C,h,w]  d(sum_px kd_px)/d lr, kd_px = -loss_px
-  float* sums;          // [3] {sum ce_px, #non-ignored, sum kd_px}
+  float* g_kd;          // [B,C,h,w]  d(sum_px kd_px)/d lr, kd_px = -loss_px (unused in the CE-only form)
+  float* sums;          // [3] {sum ce_px, #non-ignored, sum kd_px} (sum kd_px = 0 in the CE-only form)
   float* psum;          // workspace [3][nblk]: per-block partial sums
   float* slab;          // workspace [nblk][ncell]: per-block gradient cells (need_grad)
   int B, C, C_old, h, w, H, W, old_cl, ignore_index;
@@ -45,19 +47,21 @@ struct FusedArgs {
   int need_grad;
 };
 
-// dynamic smem: u[(C + C_old)][2][TX] | abuf[kChunkC][4][kRG][TX] | xw0[TX] xw1[TX] | xi0[TX] xi1[TX] | rng[ncx][4]
+// dynamic smem: u[(C + C_old)][2][TX] | abuf[kChunkC][2 NT][kRG][TX] | xw0[TX] xw1[TX] | xi0[TX] xi1[TX] | rng[ncx][4]
 constexpr int kChunkC = 8;   // channels per x-reduction pass (4: 0.562 ms, 8: 0.518 ms, 16: 0.536 ms at the bench shape)
-template <int TX>
+// KD: the CE + KD form; false: the CE-only form (a.C_old == 0, a.lo, a.g_kd unused).  NT gradient terms per cell.
+template <int TX, bool KD>
 __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, int ncx_cap) {
   extern __shared__ __align__(16) float fs[];
   constexpr int NW = TX * kRG / 32;
-  const int C = a.C, Co = a.C_old, CT = C + Co;
+  constexpr int NT = KD ? 2 : 1;
+  const int C = a.C, Co = KD ? a.C_old : 0, CT = C + Co;
   float* u = fs;                               // [CT][2][TX]  x-blended tap rows per column
-  // [kChunkC * 4 planes][kRG][TX] y-reduced gradient terms of one channel chunk; the plane stride is odd so that the
-  // 16 planes a warp of the x pass reads at the same (row group, column) fall into different banks
+  // [kChunkC * 2 NT planes][kRG][TX] y-reduced gradient terms of one channel chunk; the plane stride is odd so that
+  // the 16 planes a warp of the x pass reads at the same (row group, column) fall into different banks
   constexpr int PS = kRG * TX + 1;
   float* abuf = u + (size_t)CT * 2 * TX;
-  float* xw0 = abuf + kChunkC * 4 * PS + 3;  // x-tap weights of the tile's columns
+  float* xw0 = abuf + kChunkC * 2 * NT * PS + 3;  // x-tap weights of the tile's columns
   float* xw1 = xw0 + TX;
   int* xi0 = reinterpret_cast<int*>(xw1 + TX);  // tile-local low-res column of each tap (-1: column outside the image)
   int* xi1 = xi0 + TX;
@@ -87,7 +91,7 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
   const int nrow = Yb - Ya + 1;
   const int blk = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
   const int nblk = gridDim.x * gridDim.y * gridDim.z;
-  const int ncell = 2 * ncx_cap * C * 2;
+  const int ncell = 2 * ncx_cap * C * NT;
   if (nrow <= 0) {  // uniform per block (cannot happen when upsampling; kept for safety): contributes zeros
     if (threadIdx.x < 3) a.psum[(size_t)threadIdx.x * nblk + blk] = 0.f;
     if (a.need_grad)
@@ -107,7 +111,7 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
   // x-blended tap rows for every channel of this column (channels split over the row groups)
   {
     const float* pn = a.lr + (size_t)b * C * a.h * a.w;
-    const float* po = a.lo + (size_t)b * Co * a.h * a.w;
+    const float* po = KD ? a.lo + (size_t)b * Co * a.h * a.w : nullptr;
     for (int c = rg; c < CT; c += kRG) {
       const float* p = (c < C) ? pn + (size_t)c * a.h * a.w : po + (size_t)(c - C) * a.h * a.w;
       const float v00 = __ldg(p + k * a.w + tx.i0), v01 = __ldg(p + k * a.w + tx.i1);
@@ -169,9 +173,9 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
         const float x2 = x * kLog2e;
         if (c == a.old_cl) mo[q] = m[q], so[q] = s[q];  // snapshot: log-sum-exp over the first old_cl channels
         lse_push(m[q], s[q], x2);
-        if (bkg) lse_push(mb[q], sb[q], x2);
+        if (KD && bkg) lse_push(mb[q], sb[q], x2);
         picked[q] = (lab[q] == c) ? x : picked[q];
-        if (c < Co) {
+        if (KD && c < Co) {
           const float tv = __fmaf_rn(v0, h0[q], __fmul_rn(v1, h1[q])) * a2;
           if (c == 0) t0v[q] = tv;
           const float d = tv - mt[q];
@@ -200,7 +204,7 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
       if (colok) {
         ce_acc += l;
         valid_acc += ign ? 0.f : 1.f;
-        kd_acc += kdpx;
+        if (KD) kd_acc += kdpx;
       }
       // phase B sees: label -1 = no CE gradient (ignored / out of image), -2 = background-remapped pixel (its CE
       // gradient subtracts p_c exp(lse - lse_old) over the old classes; s_fold is 0 for every other pixel)
@@ -251,7 +255,7 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
   for (int c = 0; c < C; ++c) {
     const float u0 = u[((size_t)c * 2) * TX + xl], u1 = u[((size_t)c * 2 + 1) * TX + xl];
     float v0 = 0.f, v1 = 0.f;
-    if (c < Co) v0 = u[((size_t)(C + c) * 2) * TX + xl], v1 = u[((size_t)(C + c) * 2 + 1) * TX + xl];
+    if (KD && c < Co) v0 = u[((size_t)(C + c) * 2) * TX + xl], v1 = u[((size_t)(C + c) * 2 + 1) * TX + xl];
     const bool in_sb = (c == 0) || (c >= Co);
     const bool old_fg = (c >= 1) && (c < Co);
     const float oldc = (c < a.old_cl) ? 1.f : 0.f;  // uniform: channel c belongs to the old classes
@@ -266,34 +270,37 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
       // dCE/dx_c = p_c - [old c] p_c fold - [c == label]   (fold = 0 unless the pixel was remapped to background)
       const float sub = fmaf(p * oldc, s_fold[j], (c == lab) ? 1.f : 0.f);
       const float dce = (lab == -1) ? 0.f : (p - sub);
-      float dkd = p;
-      if (in_sb) dkd -= p * s_fb[j];
-      if (old_fg) dkd -= ex2f(fmaf(__fmaf_rn(v0, h0, __fmul_rn(v1, h1)), a2, -s_lt2[j]));
-      dkd *= inv_co;
       ce0 = fmaf(h0, dce, ce0);
       ce1 = fmaf(h1, dce, ce1);
-      kd0 = fmaf(h0, dkd, kd0);
-      kd1 = fmaf(h1, dkd, kd1);
+      if (KD) {
+        float dkd = p;
+        if (in_sb) dkd -= p * s_fb[j];
+        if (old_fg) dkd -= ex2f(fmaf(__fmaf_rn(v0, h0, __fmul_rn(v1, h1)), a2, -s_lt2[j]));
+        dkd *= inv_co;
+        kd0 = fmaf(h0, dkd, kd0);
+        kd1 = fmaf(h1, dkd, kd1);
+      }
     }
     // park the four y-reduced terms of this channel; every kChunkC channels one thread per cell folds the x taps
     {
       const int cl = c % kChunkC;
-      float* ab = abuf + (size_t)cl * 4 * PS + rg * TX + xl;
-      ab[0] = ce0, ab[PS] = ce1, ab[2 * PS] = kd0, ab[3 * PS] = kd1;
+      float* ab = abuf + (size_t)cl * 2 * NT * PS + rg * TX + xl;
+      ab[0] = ce0, ab[PS] = ce1;
+      if (KD) ab[2 * PS] = kd0, ab[3 * PS] = kd1;
     }
     if ((c + 1) % kChunkC == 0 || c == C - 1) {
       const int c_first = c - (c % kChunkC);
       __syncthreads();
       // work item = (output cell value, tap side): adjacent lanes take the i0 / i1 column range of one output and
       // exchange their partial sums; four row-group chains per thread keep the FMA pipe busy
-      const int n_out = 2 * ncx_cap * kChunkC * 2;  // (yy, cx, channel of the chunk, term)
+      const int n_out = 2 * ncx_cap * kChunkC * NT;  // (yy, cx, channel of the chunk, term)
       for (int w2 = threadIdx.x; w2 < ((2 * n_out + 31) & ~31); w2 += TX * kRG) {
         const int side = w2 & 1, o = w2 >> 1;
         const bool live = o < n_out;
-        const int term = o & 1, cl = (o >> 1) % kChunkC;
-        const int cx = live ? (o / (2 * kChunkC)) % ncx_cap : 0, yy = live ? (o / (2 * kChunkC)) / ncx_cap : 0;
+        const int term = KD ? o & 1 : 0, cl = (o >> (NT - 1)) % kChunkC;
+        const int cx = live ? (o / (NT * kChunkC)) % ncx_cap : 0, yy = live ? (o / (NT * kChunkC)) / ncx_cap : 0;
         const int cc = c_first + cl;
-        const float* ab = abuf + ((size_t)cl * 4 + (term * 2 + yy)) * PS;
+        const float* ab = abuf + ((size_t)cl * 2 * NT + (term * 2 + yy)) * PS;
         const float* xw = side ? xw1 : xw0;
         const int xa = live ? rng[cx * 4 + 2 * side] : 0, xb = live ? rng[cx * 4 + 2 * side + 1] : 0;
         float acc[kRG];
@@ -308,7 +315,7 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
         const float mine = (acc[0] + acc[1]) + (acc[2] + acc[3]);  // fixed order: deterministic
         const float other = __shfl_xor_sync(0xffffffffu, mine, 1);
         if (live && side == 0 && cc <= c)
-          a.slab[(size_t)blk * ncell + (((size_t)yy * ncx_cap + cx) * C + cc) * 2 + term] = mine + other;
+          a.slab[(size_t)blk * ncell + (((size_t)yy * ncx_cap + cx) * C + cc) * NT + term] = mine + other;
       }
       __syncthreads();
     }
@@ -317,11 +324,13 @@ __global__ void __launch_bounds__(TX * kRG) seg_fused_kernel(const FusedArgs a, 
 
 // Second stage: fixed-order sums of the per-block slabs.  One thread per low-res element (b, c, gy, gx), both terms.
 // Sources of row gy: interval gy as its upper tap row (yy = 0), interval gy-1 as its lower tap row (yy = 1), and - at
-// the bottom border, where the lower tap is clamped - interval h-1's lower tap row again.
+// the bottom border, where the lower tap is clamped - interval h-1's lower tap row again.  KD = false: dCE only.
+template <bool KD>
 __global__ void __launch_bounds__(256)
 seg_fused_gather_kernel(const FusedArgs a, int TX, int ntx, int ncx_cap) {
+  constexpr int NT = KD ? 2 : 1;
   const int C = a.C;
-  const size_t ncell = (size_t)2 * ncx_cap * C * 2;
+  const size_t ncell = (size_t)2 * ncx_cap * C * NT;
   const long long n = (long long)a.B * C * a.h * a.w;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const int gx = (int)(i % a.w), gy = (int)((i / a.w) % a.h);
@@ -337,12 +346,16 @@ seg_fused_gather_kernel(const FusedArgs a, int TX, int ntx, int ncx_cap) {
         const int cx = gx - bilinear_tap(min(t * TX, a.W - 1), a.scale_w, a.w, a.W).i0;
         if (cx < 0 || cx >= ncx_cap) continue;
         const size_t blk = ((size_t)b * a.h + k) * ntx + t;
-        const float2 v = *reinterpret_cast<const float2*>(a.slab + blk * ncell + (((size_t)yy * ncx_cap + cx) * C + c) * 2);
-        ce += v.x, kd += v.y;
+        if (KD) {
+          const float2 v = *reinterpret_cast<const float2*>(a.slab + blk * ncell + (((size_t)yy * ncx_cap + cx) * C + c) * 2);
+          ce += v.x, kd += v.y;
+        } else {
+          ce += a.slab[blk * ncell + ((size_t)yy * ncx_cap + cx) * C + c];
+        }
       }
     }
     a.g_ce[i] = ce;
-    a.g_kd[i] = kd;
+    if (KD) a.g_kd[i] = kd;
   }
 }
 
@@ -363,13 +376,14 @@ struct FusedPlan {
   size_t ncell, floats;  // workspace: psum [3][nblk] (padded to 4 floats) then slab [nblk][ncell]
 };
 
+// C_old == 0 plans the CE-only form: one gradient term per cell instead of two
 static bool fused_plan(int B, int C, int C_old, int h, int w, int W, FusedPlan& p) {
   // column tile: the widest of {128, 64, 32} whose shared memory fits
-  const int CT = C + C_old;
+  const int CT = C + C_old, NT = C_old > 0 ? 2 : 1;
   p.TX = 0;
   for (int cand : {128, 64, 32}) {
     const int ncx = (int)((double)cand * w / W) + 3;
-    const size_t need = ((size_t)CT * 2 * cand + (size_t)kChunkC * 4 * (kRG * cand + 1) + 3 + 4 * (size_t)cand +
+    const size_t need = ((size_t)CT * 2 * cand + (size_t)kChunkC * 2 * NT * (kRG * cand + 1) + 3 + 4 * (size_t)cand +
                          4 * (size_t)ncx) * sizeof(float);
     if (need <= 72 * 1024 || (cand == 32 && need <= 200 * 1024)) {  // prefer >= 3 blocks per SM
       p.TX = cand, p.smem = need, p.ncx = ncx;
@@ -379,7 +393,7 @@ static bool fused_plan(int B, int C, int C_old, int h, int w, int W, FusedPlan& 
   if (p.TX == 0) return false;
   p.ntx = (W + p.TX - 1) / p.TX;
   p.nblk = (long long)B * h * p.ntx;
-  p.ncell = (size_t)2 * p.ncx * C * 2;
+  p.ncell = (size_t)2 * p.ncx * C * NT;
   p.floats = (((size_t)3 * p.nblk + 3) & ~(size_t)3) + (size_t)p.nblk * p.ncell;
   return true;
 }
@@ -391,7 +405,7 @@ using namespace ucd;
 extern "C" size_t ucd_seg_fused_workspace_floats(int B, int C, int C_old, int h, int w, int H, int W) {
   (void)H;
   FusedPlan p;
-  if (B <= 0 || C <= 0 || C_old <= 0 || h <= 0 || w <= 0 || W < w || !fused_plan(B, C, C_old, h, w, W, p)) return 0;
+  if (B <= 0 || C <= 0 || C_old < 0 || h <= 0 || w <= 0 || W < w || !fused_plan(B, C, C_old, h, w, W, p)) return 0;
   return p.floats;
 }
 
@@ -399,9 +413,10 @@ extern "C" int ucd_seg_fused_fwd(const float* lr, const float* lr_old, int64_t* 
                                  float* sums, float* workspace, size_t workspace_floats, int B, int C, int C_old, int h,
                                  int w, int H, int W, int old_cl, int ignore_index, float alpha, int need_grad,
                                  void* stream) {
-  UCD_CHECK_ARG(lr && lr_old && labels && sums && workspace, "ucd_seg_fused_fwd: null pointer");
-  UCD_CHECK_ARG(!need_grad || (g_ce && g_kd), "ucd_seg_fused_fwd: need_grad without gradient buffers");
-  UCD_CHECK_ARG(B > 0 && C > 0 && C_old >= 1 && C >= C_old && h > 0 && w > 0 && H >= h && W >= w,
+  const bool kd = C_old > 0;  // C_old == 0: the CE-only form (no old model; lr_old and g_kd are not read)
+  UCD_CHECK_ARG(lr && (lr_old || !kd) && labels && sums && workspace, "ucd_seg_fused_fwd: null pointer");
+  UCD_CHECK_ARG(!need_grad || (g_ce && (g_kd || !kd)), "ucd_seg_fused_fwd: need_grad without gradient buffers");
+  UCD_CHECK_ARG(B > 0 && C > 0 && C_old >= 0 && C >= C_old && h > 0 && w > 0 && H >= h && W >= w,
                 "ucd_seg_fused_fwd: bad shape (upsampling only)");
   UCD_CHECK_ARG(old_cl >= 0 && old_cl <= C, "ucd_seg_fused_fwd: old_cl outside [0,C]");
   UCD_CHECK_ARG(B <= 65535 && h <= 65535, "ucd_seg_fused_fwd: batch / rows too large for the grid");
@@ -423,20 +438,29 @@ extern "C" int ucd_seg_fused_fwd(const float* lr, const float* lr_old, int64_t* 
   const size_t smem = p.smem;
   cudaError_t e;
   dim3 grid(p.ntx, h, B);
-#define UCD_LAUNCH_FUSED(T)                                                                                          \
+#define UCD_LAUNCH_FUSED(T, K)                                                                                       \
   do {                                                                                                               \
     if (smem > 48 * 1024) {                                                                                          \
-      e = cudaFuncSetAttribute(seg_fused_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);         \
+      e = cudaFuncSetAttribute(seg_fused_kernel<T, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);      \
       if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(seg_fused_kernel)");                           \
     }                                                                                                                \
-    seg_fused_kernel<T><<<grid, T * kRG, smem, st>>>(a, ncx);                                                    \
+    seg_fused_kernel<T, K><<<grid, T * kRG, smem, st>>>(a, ncx);                                                     \
   } while (0)
-  if (TX == 128)
-    UCD_LAUNCH_FUSED(128);
-  else if (TX == 64)
-    UCD_LAUNCH_FUSED(64);
-  else
-    UCD_LAUNCH_FUSED(32);
+  if (kd) {
+    if (TX == 128)
+      UCD_LAUNCH_FUSED(128, true);
+    else if (TX == 64)
+      UCD_LAUNCH_FUSED(64, true);
+    else
+      UCD_LAUNCH_FUSED(32, true);
+  } else {
+    if (TX == 128)
+      UCD_LAUNCH_FUSED(128, false);
+    else if (TX == 64)
+      UCD_LAUNCH_FUSED(64, false);
+    else
+      UCD_LAUNCH_FUSED(32, false);
+  }
 #undef UCD_LAUNCH_FUSED
   UCD_CHECK_LAUNCH("seg_fused_kernel");
   seg_fused_sums_kernel<<<3, 1024, 0, st>>>(a.psum, (int)p.nblk, sums);
@@ -445,7 +469,10 @@ extern "C" int ucd_seg_fused_fwd(const float* lr, const float* lr_old, int64_t* 
     const long long n = (long long)B * C * h * w;
     long long blocks = (n + 255) / 256;
     if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-    seg_fused_gather_kernel<<<(unsigned)blocks, 256, 0, st>>>(a, TX, p.ntx, ncx);
+    if (kd)
+      seg_fused_gather_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(a, TX, p.ntx, ncx);
+    else
+      seg_fused_gather_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(a, TX, p.ntx, ncx);
     UCD_CHECK_LAUNCH("seg_fused_gather_kernel");
   }
   return UCD_OK;

@@ -395,6 +395,63 @@ upsample_bwd_sweep_kernel(const float* __restrict__ gout, float* __restrict__ gi
   }
 }
 
+// Prediction without the upsample: pred[b,Y,X] = argmax over c of the value ucd_upsample_bilinear_fwd writes at
+// [b,c,Y,X], bit for bit: the same taps and the same bilinear_blend operation order (SMALL: ATen's small-output order,
+// H + W <= 128), ties to the first maximal channel, NaN maximal (torch.argmax).  block = (image, low-res row interval
+// k, column tile); thread (x, g) owns column x and rows g, g + kArgRG, ... of the interval, kArgRPT of them per pass
+// (intervals longer than kArgRG * kArgRPT rows, i.e. scale factors above ~30, take more passes).  Channels are the
+// outer loop: the column's 2x2 source cell is loaded once per channel and every row of the thread updates a running
+// (max, index) held in registers.  Only the int64 prediction is written.
+constexpr int kArgTX = 64, kArgRG = 4, kArgRPT = 8;
+template <bool SMALL>
+__global__ void __launch_bounds__(kArgTX * kArgRG)
+upsample_argmax_kernel(const float* __restrict__ in, int64_t* __restrict__ pred, int C, int h, int w, int H, int W,
+                       float scale_h, float scale_w) {
+  __shared__ int s_ya, s_yb;
+  const int b = blockIdx.z, k = blockIdx.y;
+  const int xl = threadIdx.x % kArgTX, rg = threadIdx.x / kArgTX;  // rg is warp-uniform
+  const int X = blockIdx.x * kArgTX + xl;
+  // rows of this interval: all Y with tap.i0 == k (contiguous), found in a conservative candidate range
+  if (threadIdx.x == 0) s_ya = H, s_yb = -1;
+  __syncthreads();
+  const float inv = (float)H / (float)h;
+  const int lo = max((int)floorf(((float)k - 0.5f) * inv) - 2, 0);
+  const int hi = min((int)ceilf(((float)k + 1.5f) * inv) + 2, H - 1);
+  for (int Y = lo + (int)threadIdx.x; Y <= hi; Y += blockDim.x)
+    if (bilinear_tap(Y, scale_h, h, H).i0 == k) atomicMin(&s_ya, Y), atomicMax(&s_yb, Y);
+  __syncthreads();
+  const int Ya = s_ya, nrow = s_yb - s_ya + 1;
+  if (nrow <= 0 || X >= W) return;
+  const Tap tx = bilinear_tap(X, scale_w, w, W);
+  const int k1 = min(k + 1, h - 1);  // = the lower tap of every row of the interval
+  const int o00 = k * w + tx.i0, o01 = k * w + tx.i1, o10 = k1 * w + tx.i0, o11 = k1 * w + tx.i1;
+  const size_t plane = (size_t)h * w;
+  const float* src = in + (size_t)b * C * plane;
+  for (int r0 = rg; r0 < nrow; r0 += kArgRG * kArgRPT) {
+    const int nj = (nrow - r0 + kArgRG - 1) / kArgRG;  // rows of this thread in this pass (warp-uniform)
+    float h0[kArgRPT], h1[kArgRPT], best[kArgRPT];
+    int arg[kArgRPT];
+#pragma unroll
+    for (int j = 0; j < kArgRPT; ++j) {
+      const Tap ty = bilinear_tap(Ya + min(r0 + j * kArgRG, nrow - 1), scale_h, h, H);
+      h0[j] = ty.w0, h1[j] = ty.w1, best[j] = -INFINITY, arg[j] = 0;
+    }
+    const float* p = src;
+    for (int c = 0; c < C; ++c, p += plane) {
+      const float v00 = __ldg(p + o00), v01 = __ldg(p + o01), v10 = __ldg(p + o10), v11 = __ldg(p + o11);
+#pragma unroll
+      for (int j = 0; j < kArgRPT; ++j) {
+        if (!SMALL && j >= nj) break;  // (with this exit the SMALL form, 4 weight products per row, spills registers)
+        const float v = bilinear_blend(SMALL, v00, v01, v10, v11, h0[j], h1[j], tx.w0, tx.w1);
+        if (j < nj && (v > best[j] || (isnan(v) && !isnan(best[j])))) best[j] = v, arg[j] = c;
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < kArgRPT; ++j)
+      if (j < nj) pred[((size_t)b * H + Ya + r0 + j * kArgRG) * W + X] = arg[j];
+  }
+}
+
 }  // namespace ucd
 
 using namespace ucd;
@@ -507,5 +564,22 @@ extern "C" int ucd_upsample_bilinear_bwd(const float* gout, float* gin, int64_t 
                                          (float)H / (float)h, (float)W / (float)w, ny_cap);
     UCD_CHECK_LAUNCH("upsample_bwd_kernel");
   }
+  return UCD_OK;
+}
+
+extern "C" int ucd_upsample_argmax(const float* lr, int64_t* pred, int B, int C, int h, int w, int H, int W,
+                                   void* stream) {
+  UCD_CHECK_ARG(lr && pred, "ucd_upsample_argmax: null pointer");
+  UCD_CHECK_ARG(B > 0 && C > 0 && h > 0 && w > 0 && H >= h && W >= w, "ucd_upsample_argmax: bad shape (upsampling only)");
+  UCD_CHECK_ARG(B <= 65535 && h <= 65535, "ucd_upsample_argmax: batch / rows too large for the grid");
+  UCD_CHECK_ARG((long long)h * w < (1ll << 30), "ucd_upsample_argmax: source plane too large");
+  cudaStream_t st = (cudaStream_t)stream;
+  const float sh = (float)h / (float)H, sw = (float)w / (float)W;
+  dim3 grid((W + kArgTX - 1) / kArgTX, h, B);
+  if (H + W <= 128)  // the operation order ucd_upsample_bilinear_fwd uses at this size
+    upsample_argmax_kernel<true><<<grid, kArgTX * kArgRG, 0, st>>>(lr, pred, C, h, w, H, W, sh, sw);
+  else
+    upsample_argmax_kernel<false><<<grid, kArgTX * kArgRG, 0, st>>>(lr, pred, C, h, w, H, W, sh, sw);
+  UCD_CHECK_LAUNCH("upsample_argmax_kernel");
   return UCD_OK;
 }

@@ -12,7 +12,8 @@ Same class names, constructor and ``forward`` signatures as the reference so tha
 * siblings on the same kernels (SURVEY 8f N3): ``KnowledgeDistillationLoss`` (loss.py:112-136),
   ``MaskKnowledgeDistillationLoss`` (:218-256), ``MaskCrossEntropy`` (:186-216)
 
-Opt-in, beyond the drop-in surface: ``FusedUnbiasedLosses`` (N1: upsample + UNCE + UNKD from the low-res logits),
+Opt-in, beyond the drop-in surface: ``FusedUnbiasedLosses`` (N1: upsample + UNCE + UNKD from the low-res logits; CE
+only at the base step), ``predict_bilinear`` (the argmax prediction of the upsampled logits, without the upsample),
 ``PixelContrastiveDistillation`` (N4: prep + contrastive loss without the 5-tuple, no host sync, CUDA-graph capturable).
 
 Everything runs in hand-written sm_100a CUDA kernels behind the C ABI of include/ucd_b200.h
@@ -104,6 +105,24 @@ def interpolate_bilinear(x, size):
     if out.requires_grad:   # where `out` came from, for a loss chain that folds the adjoint into its backward (_Route)
         out._ucd_upsample = (x, x._version, out._version)
     return out
+
+
+@torch.no_grad()
+def predict_bilinear(logits_lr, size):
+    """``interpolate_bilinear(logits_lr, size).max(dim=1)[1]`` - the int64 [B,H,W] prediction of validation and test -
+    without the [B,C,H,W] upsample: one kernel interpolates every channel on the fly and keeps a running argmax per
+    pixel.  Bit-identical to the argmax of ``interpolate_bilinear`` (ties to the first channel, NaN maximal, as
+    ``torch.argmax``).  Upsampling only; no autograd."""
+    _need_cuda(logits_lr)
+    if logits_lr.dim() != 4:
+        raise ValueError("predict_bilinear: logits must be [B,C,h,w]")
+    x = _f32c(logits_lr)
+    B, C, h, w = x.shape
+    H, W = int(size[0]), int(size[1])
+    pred = torch.empty(B, H, W, device=x.device, dtype=torch.int64)
+    if pred.numel() > 0:
+        check(_lib.lib().ucd_upsample_argmax(ptr(x), ptr(pred), B, C, h, w, H, W, cur_stream()), "upsample_argmax")
+    return pred
 
 
 class _Route:
@@ -1253,22 +1272,24 @@ class PixelContrastiveDistillation(nn.Module):
 # ----------------------------------------------------------------------------------------------
 class _SegFusedFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, lr, lr_old, labels, old_cl, ignore_index, alpha):
+    def forward(ctx, lr, lr_old, labels, old_cl, ignore_index, alpha, grad_enabled):
         _need_cuda(lr, lr_old, labels)
-        x, t = _f32c(lr), _f32c(lr_old)
+        x = _f32c(lr)
+        t = None if lr_old is None else _f32c(lr_old)   # None: the CE-only form (C_old = 0, the kd sum is 0)
         B, C, h, w = x.shape
-        C_old = t.shape[1]
+        C_old = 0 if t is None else t.shape[1]
         H, W = labels.shape[-2:]
         dev = x.device
-        need_grad = bool(ctx.needs_input_grad[0])
+        # needs_input_grad only sees requires_grad: under no_grad no gradient buffer is allocated or written
+        need_grad = bool(ctx.needs_input_grad[0]) and grad_enabled
         sums = torch.empty(3, device=dev, dtype=torch.float32)
-        g = torch.empty(2, B, C, h, w, device=dev, dtype=torch.float32) if need_grad else None
+        g = torch.empty(2 if t is not None else 1, B, C, h, w, device=dev, dtype=torch.float32) if need_grad else None
         n_ws = int(_lib.lib().ucd_seg_fused_workspace_floats(B, C, C_old, h, w, H, W))
         if n_ws == 0:
             raise ValueError("FusedUnbiasedLosses: shapes not supported (%s)" % ((B, C, C_old, h, w, H, W),))
         ws = torch.empty(n_ws, device=dev, dtype=torch.float32)
         check(_lib.lib().ucd_seg_fused_fwd(ptr(x), ptr(t), ptr(labels), ptr(g[0]) if need_grad else None,
-                                           ptr(g[1]) if need_grad else None, ptr(sums), ptr(ws), n_ws, B, C, C_old,
+                                           ptr(g[1]) if need_grad and t is not None else None, ptr(sums), ptr(ws), n_ws, B, C, C_old,
                                            h, w, H, W, old_cl, ignore_index, float(alpha), 1 if need_grad else 0,
                                            cur_stream()), "seg_fused_fwd")
         ctx.save_for_backward(g)
@@ -1279,8 +1300,10 @@ class _SegFusedFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_ce, g_kd, _g_cnt):
         (g,) = ctx.saved_tensors
-        d = g[0] * (g_ce / ctx.n_px) + g[1] * (g_kd / ctx.n_px)   # two [B,C,h,w] tensors: negligible
-        return d.to(ctx.in_dtype), None, None, None, None, None
+        d = g[0] * (g_ce / ctx.n_px)
+        if g.shape[0] == 2:
+            d = d + g[1] * (g_kd / ctx.n_px)   # two [B,C,h,w] tensors: negligible
+        return d.to(ctx.in_dtype), None, None, None, None, None, None
 
 
 class FusedUnbiasedLosses(nn.Module):
@@ -1295,6 +1318,14 @@ class FusedUnbiasedLosses(nn.Module):
     ``ce`` averages over ALL pixels of the batch (the trainer's ``.mean()`` of the 'none'-reduced loss);
     ``ce_reduction='valid'`` divides by the number of non-ignored pixels instead (nll_loss 'mean').
     Labels are remapped in place like ``UnbiasedCrossEntropy`` does.
+
+    The base step has no old model: ``FusedUnbiasedLosses(0)(out_lowres, None, labels)`` returns ``(ce, None)``,
+    computed by the CE-only form of the kernel.  With ``old_cl=0`` the unbiased CE is plain cross-entropy: for labels
+    in [0, C) and ``ignore_index >= 0`` it equals ``F.cross_entropy(interpolate(lr), labels, ignore_index=ii,
+    reduction='none').mean()`` ('valid': nll 'mean').  This relies on the kernels' reading of ``old_cl=0``, which
+    ``UnbiasedCrossEntropy(old_cl=0)`` shares: the background branch needs ``old_cl > 0``.  (The reference's
+    log-sum-exp over zero old channels would make label-0 pixels +inf.)  As in ``UnbiasedCrossEntropy``, labels below
+    ``old_cl`` - negative ones included - are remapped to 0 in place, so a negative ``ignore_index`` is not ignored.
     """
 
     def __init__(self, old_cl, ignore_index=255, alpha=1., ce_reduction='mean'):
@@ -1304,13 +1335,18 @@ class FusedUnbiasedLosses(nn.Module):
     def forward(self, logits_lr, logits_old_lr, labels):
         if labels.dtype != torch.int64 or labels.dim() != 3:
             raise TypeError("FusedUnbiasedLosses: labels must be int64 [B,H,W]")
-        if logits_lr.dim() != 4 or logits_old_lr.dim() != 4 or logits_lr.shape[0] != labels.shape[0] \
+        if logits_old_lr is None:   # base step: the CE-only form
+            if logits_lr.dim() != 4 or logits_lr.shape[0] != labels.shape[0]:
+                raise ValueError("FusedUnbiasedLosses: logits [B,C,h,w] / labels [B,H,W] disagree")
+        elif logits_lr.dim() != 4 or logits_old_lr.dim() != 4 or logits_lr.shape[0] != labels.shape[0] \
                 or logits_lr.shape[2:] != logits_old_lr.shape[2:] or logits_old_lr.shape[1] > logits_lr.shape[1]:
             raise ValueError("FusedUnbiasedLosses: logits [B,C,h,w] / old logits [B,C_old,h,w] / labels [B,H,W] disagree")
+        old = None if logits_old_lr is None else logits_old_lr.detach()
         tgt = labels if labels.is_contiguous() else labels.contiguous()
-        ce, kd, cnt = _SegFusedFn.apply(logits_lr, logits_old_lr.detach(), tgt, self.old_cl, self.ignore_index, self.alpha)
+        ce, kd, cnt = _SegFusedFn.apply(logits_lr, old, tgt, self.old_cl, self.ignore_index, self.alpha,
+                                        torch.is_grad_enabled())
         if tgt is not labels:
             labels.copy_(tgt)
         if self.ce_reduction == 'valid':
             ce = ce * (float(labels.numel()) / cnt)
-        return ce, kd
+        return ce, (None if old is None else kd)
