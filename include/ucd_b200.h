@@ -259,6 +259,24 @@ int ucd_con_fwd(const void* feat_tiles, const void* prob_tiles, const int32_t* l
                 int64_t ldp, float inv_temperature, int need_grad, float* out, float* grad_unit,
                 void* workspace, size_t workspace_bytes, int64_t max_row_tiles, int64_t plan_row_tiles,
                 void* stream);
+/* Gradient of PixelConLossV2 with respect to the contrast features, utils/loss.py:445-466 (the reference back-propagates
+ * into contrast_feature whenever it carries a graph; SURVEY.md Appendix A.2, column side):
+ *   G_ij = dL/ds_ij = -kappa_i w_ij neg_i / den_ij (positive pair) | +kappa_i T_i exp(s_ij) (negative pair) | 0 (j is i)
+ *   grad_unit [chunk_tiles*128, 256] = d(sum_i loss_i)/d c_j = (1/tau) sum_i (M G_ij) a_i,   kappa_i = [num_i != 0]/(M num_i)
+ * (rows >= N_c are 0; scaled by g / out[1] in ucd_con_bwd with n_rows = device {N_c}, row_ref = NULL).  Call it after
+ * ucd_con_fwd (part 0, any need_grad) on the same workspace, sized by ucd_con_contrast_grad_workspace_bytes with the
+ * forward's max_row_tiles / chunk_tiles / plan_row_tiles, with the forward's column and row arguments: it reads the
+ * forward's statistics (row max, neg, num, T) and runs a transposed third sweep (contrast tiles as rows, anchor tiles
+ * streamed) that forms G pair by pair and accumulates G^T A on the tensor cores.  Single-chunk layout only
+ * (n_chunks = 1, chunk_stride_bytes = 0), p_mode 0 or 2, self_tile0 0 or -1; anything else is UCD_EINVAL.  The self
+ * pair (anchor i, column i) is never a positive; it is a negative when its two labels differ, as in the forward. */
+size_t ucd_con_contrast_grad_workspace_bytes(int64_t max_row_tiles, int64_t chunk_tiles, int64_t plan_row_tiles);
+int ucd_con_contrast_grad(const void* feat_tiles, const int32_t* lab_tiles, const int32_t* chunk_counts, int n_chunks,
+                          int64_t chunk_tiles, int64_t chunk_stride_bytes, const void* row_feat_tiles,
+                          const int32_t* row_lab_tiles, const int32_t* n_rows, const int32_t* tile_range,
+                          const int32_t* row_range, int64_t self_tile0, int p_mode, const float* dense_p, int64_t ldp,
+                          float inv_temperature, float* grad_unit, void* workspace, size_t workspace_bytes,
+                          int64_t max_row_tiles, int64_t plan_row_tiles, void* stream);
 /* Self-contrast losses of utils/loss_new.py on the same sweeps (SURVEY.md row N3):
  *   mode 0  PixelConLoss (v1), loss_new.py:354-400:  s = F F^T / tau, unshifted exponentials,
  *           loss = mean_{num_i != 0} -(1/num_i) sum_j mp_ij [s_ij - log(exp(s_ij) + neg_j)]

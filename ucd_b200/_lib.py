@@ -58,6 +58,9 @@ _PROTOS = {
     "ucd_con_fwd": (c_int, [P, P, P, P, c_int, c_int64, c_int64, c_int, c_int, P, P, P, P, P, P, c_int64, P, c_int, c_int,
                             P, c_int64, c_float, c_int, P, P, P, c_size_t, c_int64, c_int64, P]),
     "ucd_con_bwd": (c_int, [P, P, P, c_float, P, P, P, c_int64, P]),
+    "ucd_con_contrast_grad_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
+    "ucd_con_contrast_grad": (c_int, [P, P, P, c_int, c_int64, c_int64, P, P, P, P, P, c_int64, c_int, P, c_int64,
+                                      c_float, P, P, c_size_t, c_int64, c_int64, P]),
     "ucd_selfcon_workspace_bytes": (c_size_t, [c_int64]),
     "ucd_selfcon_fwd": (c_int, [P, P, P, P, P, c_int64, c_int64, c_int, c_float, c_float, c_int, P, P, P, c_size_t, P]),
 }

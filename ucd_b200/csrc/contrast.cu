@@ -15,7 +15,9 @@
 //            in bf16 -> a separate E region of tensor memory -> V += E C (tcgen05 TS with the SAME C tile read MN-major).
 //   sweep 2: S again and P = pA pC^T (K = padded C_old) -> epilogue: den, log, weights, L_i, T_i;
 //            Ucoef in bf16 -> the consumed P columns -> U += Ucoef C.
-// The gradient needs no third sweep: backward is a scaled copy of (T V - U)/(tau num).
+// The anchor gradient needs no third sweep: backward is a scaled copy of (T V - U)/(tau num).  The contrast gradient
+// (PixelConLossV2(contrast_grad=True), ucd_con_contrast_grad) does: dL/dc_j = (1/tau) sum_i G_ij a_i is the transposed
+// problem, a third sweep with the contrast columns as rows and the anchors streamed (sweep3c_cols).
 //
 // CTA = one 128-row block x one contiguous range of column tiles ("split").  Warp roles: warp 0 issues
 // bulk async copies (TMA engine) of pre-tiled bf16 operands, warp 1 owns TMEM and issues the S (and P) MMAs,
@@ -126,7 +128,7 @@ struct ConArgs {
   long long* trace;    // debug: [grid][16] cycle counters per role (ucd_con_debug_trace), or NULL
   // self-contrast losses (PixelConLoss v1 / SupConLoss, utils/loss_new.py:263-400; see sweep3_cols)
   int shift;           // sweep 2: 1 = PixelConLossV2's exp(s - m) in the denominator, 0 = unshifted (v1)
-  const float* col_a;  // sweep 3: per-pixel coefficients in column (= row) order, see sweep3_cols
+  const float* col_a;  // sweep 3: per-pixel coefficients in column (= row) order, see sweep3_cols / sweep3c_cols
   const float* col_b;
   const float* col_c;
 };
@@ -224,7 +226,9 @@ __device__ __forceinline__ void sweep1_cols(const uint32_t (&r)[32], const int* 
         cnt = ok ? cnt : 0.f;
         mv = ok ? acc : -3.0e38f;
       }
-      if (SELF) cnt -= (col == rself) ? 1.f : 0.f;
+      // the self column only counts when it exists: a row past the last column (N_a > N_c) meets col == rself in the
+      // padding of the last column tile
+      if (SELF) cnt -= (col == rself && (FULL || col < nv)) ? 1.f : 0.f;
       mx = fmaxf(mx, mv);
       neg += ev;
       num += cnt;
@@ -386,6 +390,43 @@ __device__ __forceinline__ void sweep3_cols(const uint32_t (&r)[32], const int* 
         v = same ? v - (row_c + bs[u]) : v;  // a_j differs from a_i when only some rows are anchors ('one' mode)
       }
       h[u] = (col < nv && col != rself) ? v : 0.f;
+    }
+    pk[j4 / 2] = bf16x2_bits(h[0], h[1]);
+    pk[j4 / 2 + 1] = bf16x2_bits(h[2], h[3]);
+  }
+}
+
+// ---- sweep 3, PixelConLossV2 contrast side (MODE 2: P == 1, MODE 3: dense P) on 32 columns -------------------------
+// dL/dc_j = (1/tau) sum_i G_ij a_i is the transposed problem: the CTA's rows are contrast columns j, the streamed tiles
+// are anchor rows i, and H_ji = G_ij = dL/ds_ij (SURVEY.md Appendix A.2; the common 1/M is applied by ucd_con_bwd):
+//   negative pair (la_i != lc_j):               kT_i exp(s_ij)                          kT_i = [num_i != 0] T_i / num_i
+//   positive pair (equal labels, j is not i):  -k_i P_ij neg_i / (exp(s_ij - m_i) + neg_i)    k_i = [num_i != 0] / num_i
+// The anchors' statistics come from the forward in column (= anchor) order, one float4 {kT_i, k_i, neg_i, raw row max}
+// per anchor (con_colcoef_kernel).  One ex2 per pair: its argument is s_ij for a negative and s_ij - m_i for a positive.  The
+// self pair (j == i, self_tile0 = 0) is never a positive and is a negative when its labels differ, as in sweeps 1 and 2;
+// padding rows come with nv = 0.  neg_i = 0 gives 0 for a positive pair, not NaN.  Dense P is read as P[i * ldp + j]
+// (dp points at column j of anchor row 0 of the tile): consecutive lanes read consecutive j.
+template <bool DENSE_P>
+__device__ __forceinline__ void sweep3c_cols(const uint32_t (&r)[32], const int* __restrict__ lab, int cbase, int nv, int la,
+                                             int rself, float sc, const float4* __restrict__ coef,
+                                             const float* __restrict__ dp, int ldp, uint32_t (&pk)[16]) {
+#pragma unroll
+  for (int j4 = 0; j4 < 32; j4 += 4) {
+    const int4 l4 = *reinterpret_cast<const int4*>(lab + cbase + j4);
+    const int ls[4] = {l4.x, l4.y, l4.z, l4.w};
+    float h[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int col = cbase + j4 + u;
+      const float4 q = __ldg(coef + col);  // {kT_i, k_i, neg_i, raw max of row i}
+      const float acc = __uint_as_float(r[j4 + u]);
+      const bool same = ls[u] == la;
+      const bool pos = same && col != rself;  // the self pair is a negative when its labels differ, else nothing
+      const float x = ex2f((same ? acc - q.w : acc) * sc);  // exp(s_ij - m_i) | exp(s_ij)
+      float kw = q.y;
+      if (DENSE_P) kw *= (pos && col < nv) ? __ldg(dp + col * ldp) : 0.f;  // col * ldp < 2^31 (ldp < 2^24)
+      const float v = same ? -kw * q.z * rcpf(fmaxf(x + q.z, 1e-30f)) : q.x * x;
+      h[u] = (col < nv && (pos || !same)) ? v : 0.f;
     }
     pk[j4 / 2] = bf16x2_bits(h[0], h[1]);
     pk[j4 / 2 + 1] = bf16x2_bits(h[2], h[3]);
@@ -733,7 +774,7 @@ __global__ void __launch_bounds__(kConThreads, 1) con_sweep_kernel(const ConArgs
     int thr = 0x7fffffff;
     bool warp_series = false;
     float row_a = 0.f, row_b = 0.f, row_c = 0.f;  // sweep 3: this pixel's coefficients
-    if (PHASE == 3 && grow < n_rows) row_a = a.col_a[grow], row_b = a.col_b[grow], row_c = a.col_c[grow];
+    if (PHASE == 3 && PMODE < 2 && grow < n_rows) row_a = a.col_a[grow], row_b = a.col_b[grow], row_c = a.col_c[grow];
     if (PHASE == 2) {
       rc.mraw = a.shift ? a.stats[grow] : 0.f;
       rc.negi = a.stats[a.rows_pad + grow];
@@ -766,7 +807,7 @@ __global__ void __launch_bounds__(kConThreads, 1) con_sweep_kernel(const ConArgs
       const bool full = loc.nvalid == 128;
       const bool self = loc.gtile == self_tile;
       const int* lab = reinterpret_cast<const int*>(smem + OFF_LAB + (t % 3) * 512);
-      const float* dp = (PMODE == 2) ? a.dense_p + (size_t)min(grow, (long long)n_rows - 1) * a.ldp + loc.dcol0 : nullptr;
+      const float* dp = (PHASE == 2 && PMODE == 2) ? a.dense_p + (size_t)min(grow, (long long)n_rows - 1) * a.ldp + loc.dcol0 : nullptr;
       const bool all_neg = PHASE == 1 && full && !((mword >> (tt & 31)) & 1u);
       mbar_wait_t(BAR(BAR_SF + sb), t & 1, w_sf);
       tc_fence_after();
@@ -787,7 +828,13 @@ __global__ void __launch_bounds__(kConThreads, 1) con_sweep_kernel(const ConArgs
         uint32_t r0[32], r1[32];
         auto proc = [&](int cc, const uint32_t (&rv)[32]) {
           uint32_t pk[16];
-          if (PHASE == 3)
+          if (PHASE == 3 && PMODE >= 2)  // contrast side: rows are contrast columns, the tile's columns anchors
+            sweep3c_cols<PMODE == 3>(rv, lab, c0 + cc * 32, grow < n_rows ? loc.nvalid : 0, la, self ? r : -1, sc,
+                                     reinterpret_cast<const float4*>(a.col_a) + loc.dcol0,
+                                     PMODE == 3 ? a.dense_p + loc.dcol0 * a.ldp + min(grow, (long long)n_rows - 1)
+                                                : nullptr,
+                                     (int)a.ldp, pk);
+          else if (PHASE == 3)
             sweep3_cols<PMODE>(rv, lab, c0 + cc * 32, loc.nvalid, la, self ? r : -1, sc, row_a, row_b, row_c,
                                a.col_a + loc.dcol0, (PMODE == 0 ? a.col_b : a.col_c) + loc.dcol0, pk);
           else if (all_neg)
@@ -1106,6 +1153,32 @@ selfcon_grad_kernel(const float* __restrict__ v_part, int splits, long long rows
   }
 }
 
+// PixelConLossV2 contrast gradient, after ucd_con_fwd: the per-anchor coefficients of sweep3c_cols from the forward's
+// statistics, coef[i] = {kT_i, k_i, neg_i, raw row max} with k = [num != 0] / num and T summed over the sweep-2 splits in
+// the order of con_finalize_kernel, and the counts of the transposed sweep: cnt = {N_a, 0 | N_c} (its columns are the
+// anchors, its rows the contrast columns).
+__global__ void __launch_bounds__(256)
+con_colcoef_kernel(const float* __restrict__ stats, const float* __restrict__ loss_part, int splits2, long long rows_pad,
+                   const int* __restrict__ n_rows_p, const int* __restrict__ counts, float4* __restrict__ coef,
+                   int* __restrict__ cnt) {
+  const int n_rows = *n_rows_p;
+  if (blockIdx.x == 0 && threadIdx.x == 0) cnt[0] = n_rows, cnt[1] = 0, cnt[2] = counts[0] + counts[1];
+  for (long long row = (long long)blockIdx.x * blockDim.x + threadIdx.x; row < rows_pad;
+       row += (long long)gridDim.x * blockDim.x) {
+    float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (row < n_rows) {
+      const float num = stats[2 * rows_pad + row];
+      float T = 0.f;
+      for (int s = 0; s < splits2; ++s) T += loss_part[(size_t)s * 2 * rows_pad + rows_pad + row];
+      q.y = num != 0.f ? 1.f / num : 0.f;
+      q.x = q.y * T;
+      q.z = stats[rows_pad + row];
+      q.w = stats[row];
+    }
+    coef[row] = q;
+  }
+}
+
 constexpr int kFinalizeBlocks = kNumSMs * 4;
 #ifdef UCD_DEBUG_KNOBS
 static long long* g_trace = nullptr;  // debug builds only (ucd_con_debug_trace)
@@ -1380,6 +1453,90 @@ extern "C" int ucd_selfcon_fwd(const void* feat_tiles, const int32_t* lab_tiles,
   if (rc != UCD_OK) return rc;
   selfcon_grad_kernel<<<kFinalizeBlocks, 256, 0, st>>>((const float*)(ws + plan.off_v), plan.splits, plan.rows_pad, n,
                                                         inv_temperature, grad_unit);
+  UCD_CHECK_LAUNCH("selfcon_grad_kernel");
+  return UCD_OK;
+}
+
+// ---- PixelConLossV2 contrast gradient ----------------------------------------------------------------------------
+// Workspace: the forward's plan, then the anchor coefficients [rows_pad][4] and the transposed sweep's counts, then its
+// partial products [splits][contrast tiles * 128][256].
+struct CgradLayout {
+  ConPlan fwd;
+  int splits;  // column (= anchor tile) splits of the transposed sweep
+  size_t off_coef, off_cnt, off_acc, total;
+};
+
+static CgradLayout cgrad_layout(int64_t max_row_tiles, int64_t col_tiles, int64_t plan_row_tiles) {
+  CgradLayout l;
+  l.fwd = make_plan(max_row_tiles, col_tiles, plan_row_tiles, 0);
+  l.splits = choose_splits(col_tiles, max_row_tiles);
+  auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
+  l.off_coef = up(l.fwd.total);
+  l.off_cnt = up(l.off_coef + (size_t)4 * l.fwd.rows_pad * sizeof(float));
+  l.off_acc = up(l.off_cnt + 4 * sizeof(int));
+  l.total = l.off_acc + (size_t)l.splits * col_tiles * 128 * 256 * sizeof(float);
+  return l;
+}
+
+extern "C" size_t ucd_con_contrast_grad_workspace_bytes(int64_t max_row_tiles, int64_t col_tiles,
+                                                        int64_t plan_row_tiles) {
+  if (max_row_tiles <= 0 || col_tiles <= 0) return 0;
+  return cgrad_layout(max_row_tiles, col_tiles, plan_row_tiles).total;
+}
+
+extern "C" int ucd_con_contrast_grad(const void* feat_tiles, const int32_t* lab_tiles, const int32_t* chunk_counts,
+                                     int n_chunks, int64_t chunk_tiles, int64_t chunk_stride_bytes,
+                                     const void* row_feat_tiles, const int32_t* row_lab_tiles, const int32_t* n_rows,
+                                     const int32_t* tile_range, const int32_t* row_range, int64_t self_tile0, int p_mode,
+                                     const float* dense_p, int64_t ldp, float inv_temperature, float* grad_unit,
+                                     void* workspace, size_t workspace_bytes, int64_t max_row_tiles,
+                                     int64_t plan_row_tiles, void* stream) {
+  UCD_CHECK_ARG(feat_tiles && lab_tiles && chunk_counts && row_feat_tiles && row_lab_tiles && n_rows && tile_range &&
+                    row_range && grad_unit && workspace,
+                "ucd_con_contrast_grad: null pointer");
+  UCD_CHECK_ARG(n_chunks == 1 && chunk_stride_bytes == 0,
+                "ucd_con_contrast_grad: only the single-chunk layout (n_chunks = 1, chunk_stride_bytes = 0) is supported; "
+                "gathered columns would need their gradient sent back to the owning rank");
+  UCD_CHECK_ARG(p_mode == 0 || p_mode == 2,
+                "ucd_con_contrast_grad: p_mode must be 0 (P is None) or 2 (dense P); the joint-probability tiles "
+                "(p_mode 1) are not supported");
+  UCD_CHECK_ARG(p_mode == 0 || (dense_p && ldp >= 1 && ldp < (1 << 24)),
+                "ucd_con_contrast_grad: dense P needs dense_p and 1 <= ldp < 2^24");
+  UCD_CHECK_ARG(self_tile0 == 0 || self_tile0 == -1, "ucd_con_contrast_grad: self_tile0 must be 0 or -1");
+  UCD_CHECK_ARG(chunk_tiles >= 1 && max_row_tiles >= 1, "ucd_con_contrast_grad: bad tile counts");
+  UCD_CHECK_ARG(aligned16(feat_tiles) && aligned16(lab_tiles) && aligned16(row_feat_tiles) && aligned16(row_lab_tiles) &&
+                    aligned16(grad_unit),
+                "ucd_con_contrast_grad: tile and gradient buffers must be 16 B aligned");
+  UCD_CHECK_ARG(inv_temperature > 0.f, "ucd_con_contrast_grad: bad temperature");
+  const CgradLayout l = cgrad_layout(max_row_tiles, chunk_tiles, plan_row_tiles);
+  UCD_CHECK_ARG(workspace_bytes >= l.total, "ucd_con_contrast_grad: workspace too small (%zu < %zu)", workspace_bytes,
+                l.total);
+  UCD_CHECK_ARG(chunk_tiles * l.splits < (1ll << 31), "ucd_con_contrast_grad: grid too large");
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)workspace;
+  const long long rows_pad_a = l.fwd.rows_pad;
+  float* coef = (float*)(ws + l.off_coef);
+  int* cnt = (int*)(ws + l.off_cnt);
+  con_colcoef_kernel<<<(unsigned)((rows_pad_a + 255) / 256), 256, 0, st>>>(
+      (const float*)(ws + l.fwd.off_stats), (const float*)(ws + l.fwd.off_loss_part), l.fwd.splits2, rows_pad_a, n_rows,
+      chunk_counts, reinterpret_cast<float4*>(coef), cnt);
+  UCD_CHECK_LAUNCH("con_colcoef_kernel");
+  // the transposed sweep: rows = contrast tiles, streamed columns = anchor tiles
+  ConArgs a;
+  a.feat_tiles = (const __nv_bfloat16*)row_feat_tiles, a.prob_tiles = nullptr, a.lab_tiles = row_lab_tiles;
+  a.chunk_counts = cnt, a.n_chunks = 1, a.chunk_tiles = max_row_tiles, a.chunk_stride = 0, a.chunk_origin = 0;
+  a.chunk_lo = 0, a.chunk_hi = 1, a.chunk_skip = -1, a.split_base = 0;
+  a.row_feat = (const __nv_bfloat16*)feat_tiles, a.row_prob = nullptr, a.row_lab = lab_tiles, a.n_rows = cnt + 2;
+  a.tile_range = row_range, a.row_range = tile_range, a.self_tile0 = self_tile0, a.min_new = nullptr;
+  a.dense_p = dense_p, a.ldp = ldp, a.inv_tau = inv_temperature, a.splits = l.splits, a.need_grad = 1, a.kpad = 16;
+  a.rows_pad = chunk_tiles * 128;
+  a.stats_part = nullptr, a.acc_part = (float*)(ws + l.off_acc);
+  a.stats = nullptr, a.loss_part = nullptr, a.trace = nullptr, a.shift = 0;
+  a.col_a = coef, a.col_b = a.col_c = nullptr;  // [rows_pad_a] float4 {kT, k, neg, raw row max}
+  const int rc = p_mode == 0 ? launch_sweep<3, 2>(a, chunk_tiles, st) : launch_sweep<3, 3>(a, chunk_tiles, st);
+  if (rc != UCD_OK) return rc;
+  selfcon_grad_kernel<<<kFinalizeBlocks, 256, 0, st>>>(a.acc_part, l.splits, a.rows_pad, a.rows_pad, inv_temperature,
+                                                        grad_unit);
   UCD_CHECK_LAUNCH("selfcon_grad_kernel");
   return UCD_OK;
 }

@@ -910,10 +910,12 @@ def gather_contrast_columns(payload, max_tiles, kpad, group, async_op=False):
 
 class _ConFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, anchor, cols, rows, inv_tau, p_mode, dense_p, group, ddp_scale):
+    def forward(ctx, anchor, cols, rows, inv_tau, p_mode, dense_p, group, ddp_scale, contrast=None):
         """cols / rows: dicts of device buffers (see PixelConLossV2.forward).  With a process group, ``cols`` holds the
         LOCAL payload; the all-gather of all ranks' payloads is enqueued first and sweep 1 over the local columns runs
-        while it is in flight."""
+        while it is in flight.  ``contrast``: the contrast features the single-chunk ``cols`` were packed from, when
+        their gradient is wanted (compat path, PixelConLossV2(contrast_grad=True)); ucd_con_contrast_grad then forms
+        d(sum of row losses)/d contrast after the forward, on its workspace."""
         L = _lib.lib()
         dev = anchor.device
         max_row_tiles = rows["max_tiles"]
@@ -922,6 +924,7 @@ class _ConFn(torch.autograd.Function):
         need_grad = bool(ctx.needs_input_grad[0])
         grad_unit = (torch.empty(max_row_tiles * TILE, FEAT_DIM, device=dev, dtype=torch.float32)
                      if need_grad else None)
+        contrast_grad = contrast is not None and bool(ctx.needs_input_grad[8])
 
         def run(c, part, n_chunks, stride, local_chunk, self_tile0, ws, ws_bytes):
             check(L.ucd_con_fwd(ptr(c["feat"]), ptr(c["prob"]), ptr(c["lab"]), ptr(c["counts"]), n_chunks,
@@ -932,7 +935,21 @@ class _ConFn(torch.autograd.Function):
                                 ptr(grad_unit), ptr(ws), ws_bytes, max_row_tiles, plan_tiles, cur_stream()),
                   "con_fwd")
 
-        if group is None:
+        ctx.c_unit = None
+        if group is None and contrast_grad:
+            ct = cols["chunk_tiles"]
+            ws_bytes = L.ucd_con_contrast_grad_workspace_bytes(max_row_tiles, ct, plan_tiles)
+            ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+            run(cols, 0, 1, 0, -1, rows["self_tile0"], ws, ws_bytes)
+            c_unit = torch.empty(ct * TILE, FEAT_DIM, device=dev, dtype=torch.float32)
+            check(L.ucd_con_contrast_grad(ptr(cols["feat"]), ptr(cols["lab"]), ptr(cols["counts"]), 1, ct, 0,
+                                          ptr(rows["feat"]), ptr(rows["lab"]), ptr(rows["n_rows"]), ptr(cols["range"]),
+                                          ptr(rows["range"]), rows["self_tile0"], p_mode, ptr(dense_p),
+                                          0 if dense_p is None else dense_p.shape[1], inv_tau, ptr(c_unit), ptr(ws),
+                                          ws_bytes, max_row_tiles, plan_tiles, cur_stream()), "con_contrast_grad")
+            ctx.c_unit, ctx.c_counts = c_unit, cols["counts"]   # counts[0] = N_c: the rows ucd_con_bwd writes
+            ctx.n_c, ctx.c_dtype = contrast.shape[0], contrast.dtype
+        elif group is None:
             ws_bytes = L.ucd_con_workspace_bytes(max_row_tiles, cols["n_chunks"] * cols["chunk_tiles"], plan_tiles, 0)
             ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
             run(cols, 0, cols["n_chunks"], 0, -1, rows["self_tile0"], ws, ws_bytes)
@@ -971,11 +988,19 @@ class _ConFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         grad_unit, out, n_rows, row_ref = ctx.saved_tensors
+        d_contrast = None
+        if ctx.c_unit is not None:   # same scaling as the anchor side: g / M (local compat path, no DDP factor)
+            d_c = torch.empty(ctx.n_c, FEAT_DIM, device=g.device, dtype=torch.float32)
+            check(_lib.lib().ucd_con_bwd(ptr(ctx.c_unit), ptr(out), ptr(_f32c(g.reshape(1))), 1.0, ptr(ctx.c_counts),
+                                         None, ptr(d_c), ctx.n_c, cur_stream()), "con_bwd")
+            d_contrast = d_c.to(ctx.c_dtype)
+            if not ctx.needs_input_grad[0]:
+                return None, None, None, None, None, None, None, None, d_contrast
         if ctx.n_rows_addr is not None:
             n_rows = ctx.n_rows_addr
         d_anchor = torch.empty(ctx.n_a, FEAT_DIM, device=g.device, dtype=torch.float32)
         if ctx.n_a == 0:   # a rank without anchors (it only took part in the collectives)
-            return d_anchor.to(ctx.in_dtype), None, None, None, None, None, None, None
+            return d_anchor.to(ctx.in_dtype), None, None, None, None, None, None, None, None
         # With DDP averaging parameter gradients over ranks, the exact gradient of the global-batch loss needs
         # each rank's local contribution scaled by world (columns carry no gradient, loss.py:366,395).
         check(_lib.lib().ucd_con_bwd(ptr(grad_unit), ptr(out), ptr(_f32c(g.reshape(1))), float(ctx.world),
@@ -990,7 +1015,7 @@ class _ConFn(torch.autograd.Function):
             check(bwd_fn(ptr(d_anchor), ptr(pk.anchor_f32), ptr(pk.inv_norm), ptr(pk.px_meta),
                          ptr(pk.blk_meta), ptr(df), B, h, w, cur_stream()), "con_prep_bwd")
             d_anchor = df.to(ctx.in_dtype)
-        return d_anchor, None, None, None, None, None, None, None
+        return d_anchor, None, None, None, None, None, None, None, d_contrast
 
 
 class PixelConLossV2(nn.Module):
@@ -1004,10 +1029,16 @@ class PixelConLossV2(nn.Module):
 
     Extension (SURVEY.md 8e): with ``gather_negatives=True`` and an initialised process group the
     contrast columns of all ranks are all-gathered over NCCL so negatives span the global batch.
+
+    ``contrast_grad=True``: on the compat path a ``contrast_feature`` that requires grad (under grad mode) gets its
+    gradient too, as in the reference (utils/loss.py:445-466), from a third, transposed tensor-core sweep
+    (``ucd_con_contrast_grad``); ``P`` is a constant either way.  The default refuses such a contrast, because the UCD
+    prep detaches it (utils/loss.py:366).  A :class:`JointProb` ``P`` (the tuple fast path) with such a contrast raises
+    ``ValueError``.  Under ``no_grad`` or with a contrast that does not require grad the flag changes nothing.
     """
 
     def __init__(self, sample_method='none', temperature=0.07, *, gather_negatives=False, process_group=None,
-                 ddp_grad_scale=True):
+                 ddp_grad_scale=True, contrast_grad=False):
         super(PixelConLossV2, self).__init__()
         self.temperature = temperature
         self.sample_method = sample_method
@@ -1015,6 +1046,7 @@ class PixelConLossV2(nn.Module):
         self.process_group = process_group
         # under DDP's gradient averaging the exact global-batch gradient needs the local part scaled by world
         self.ddp_grad_scale = ddp_grad_scale
+        self.contrast_grad = contrast_grad   # differentiate w.r.t. contrast_feature on the compat path
         self.max_dense_bytes = 2 << 30   # largest dense P the compat fallback may materialise (see forward)
         print(temperature)  # the reference prints it on construction (utils/loss.py:410)
 
@@ -1052,8 +1084,15 @@ class PixelConLossV2(nn.Module):
                 raise RuntimeError(msg + "  Refusing: above max_dense_bytes=%d." % self.max_dense_bytes)
             warnings.warn(msg, RuntimeWarning, stacklevel=2)
             P, pack = P.dense(), None
+        want_dc = contrast_feature.requires_grad and torch.is_grad_enabled()
         if pack is not None:
             # ---- fast path: operands packed by pre_contrastive_pixel ----
+            if want_dc and self.contrast_grad:
+                # the packed columns are the pack's own (detached) copy: the gradient would be silently lost
+                raise ValueError("PixelConLossV2(contrast_grad=True): contrast_feature requires grad, but P is a "
+                                 "JointProb handle (the packed fast path), whose columns carry no gradient; the "
+                                 "contrast gradient is formed on the compat path only: pass P.dense() (or None) and "
+                                 "plain [N, 256] tensors")
             group = self._group()
             ad = pack.addr
             rows = dict(feat=ad["feat"], prob=ad["prob"], lab=ad["lab"], n_rows=ad["counts"], keep=pack.payload,
@@ -1071,13 +1110,16 @@ class PixelConLossV2(nn.Module):
             raise ValueError("PixelConLossV2: features must be [N,%d]" % FEAT_DIM)
         n_a, n_c = anchor_features.shape[0], contrast_feature.shape[0]
         if n_a == 0 or n_c == 0:
+            if want_dc and self.contrast_grad:
+                return anchor_features.sum() * 0.0 + contrast_feature.sum() * 0.0
             return anchor_features.sum() * 0.0
-        if contrast_feature.requires_grad and torch.is_grad_enabled():
+        if want_dc and not self.contrast_grad:
             # the reference back-propagates through contrast_feature when it carries a graph (utils/loss.py:445-466);
-            # the sweeps only form d loss / d anchor_features (the v2 prep detaches the contrast side, loss.py:366)
-            raise RuntimeError("PixelConLossV2: contrast_feature requires grad, but this implementation only "
+            # by default only d loss / d anchor_features is formed (the v2 prep detaches the contrast side, loss.py:366)
+            raise RuntimeError("PixelConLossV2: contrast_feature requires grad, but this module only "
                                "differentiates w.r.t. anchor_features (the UCD prep detaches the contrast side, "
-                               "utils/loss.py:366); pass contrast_feature.detach() if that is what you mean")
+                               "utils/loss.py:366); pass contrast_feature.detach() if that is what you mean, or "
+                               "construct it with contrast_grad=True")
         a32, c32 = _f32c(anchor_features.detach()), _f32c(contrast_feature.detach())
         la = anchor_labels.reshape(-1).to(device=dev, dtype=torch.int32).contiguous()
         lc = contrast_labels.reshape(-1).to(device=dev, dtype=torch.int32).contiguous()
@@ -1106,6 +1148,8 @@ class PixelConLossV2(nn.Module):
         cols = dict(feat=cfeat, prob=None, lab=clab, range=crange, counts=counts, n_chunks=1, chunk_tiles=ct, kpad=16,
                     min_new=None)
         rows = dict(feat=rfeat, prob=None, lab=rlab, range=rrange, n_rows=n_rows, max_tiles=rt, self_tile0=0)
+        if want_dc:
+            return _ConFn.apply(anchor_features, cols, rows, inv_tau, p_mode, dense_p, None, False, contrast_feature)
         return _ConFn.apply(anchor_features, cols, rows, inv_tau, p_mode, dense_p, None, False)
 
 
